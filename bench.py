@@ -4,6 +4,7 @@ neck + heads + decode + NMS) on N B200s, batch-sharded, no collective.
 
     python bench.py --gpus N --steps K --warmup W            # this build (CUDA engine)
     python bench.py --impl reference --gpus N ...             # CPU restatement of the reference
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's detections
 
 A "step" is one pass of the hot path over one batch of synthetic images.  Workload at
 every N = the configuration BASELINE.json's metric is quoted on ("416 bs256"): configs[1]'s model
@@ -28,6 +29,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the tree may be read-only; the benchmark writes nothing into it
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -45,7 +47,8 @@ CONF, NMS_T = 0.001, 0.5
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 100 for detect, 30 for train)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=BATCH)
@@ -56,6 +59,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--dump-profile", default="")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the detections of the last timed step as DIR/<name>.npy (rank 0; see dump_outputs)")
     ap.add_argument("--strong", action="store_true",
                     help="strong scaling: --batch is the TOTAL batch, split evenly over the ranks (configs[2])")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run oracle check of two images")
@@ -63,7 +68,14 @@ def parse():
     ap.add_argument("--workload", default="detect", choices=["detect", "train"],
                     help="train = BASELINE configs[4]: the data-parallel training step (tools/gpu_train_step_bench.py), "
                          "32 images per GPU unless --batch is given")
-    return ap.parse_args()
+    a = ap.parse_args()
+    if a.steps is None:
+        a.steps = 30 if a.workload == "train" else 100
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.workload != "detect" or a.impl != "b200"):
+        ap.error("--dump-outputs records the detect workload of --impl b200 only")
+    return a
 
 
 # --------------------------------------------------------------------------------------------
@@ -213,6 +225,30 @@ def latency_b1(sd, dev, size, mode):
             "by_input_size": out}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, out_dev):
+    """Writes what forward_detect handed back in the last timed step, so that two builds can be compared on the
+    same seeded inputs: `counts` [B] (detections kept per image), and for a fixed sample of the images
+    (`images`, ascending) their valid rows one after another: `boxes` [M,4], `scores` [M], `cls` [M].  Rows past
+    an image's count are not part of the result and are left out.  The sample is every image if the worst case
+    (all N candidates kept) fits DUMP_BYTES, else a seeded choice of as many images as fit; it depends only on
+    the batch and the input size.  All arrays float32 (class ids and counts are exact)."""
+    boxes, scores, cls, counts = (t.cpu().numpy() for t in out_dev)
+    batch, n = scores.shape
+    fit = max(1, (DUMP_BYTES - 8 * batch) // (n * 6 * 4))
+    images = np.arange(batch) if fit >= batch else np.sort(np.random.default_rng(0).choice(batch, fit, replace=False))
+    rows = [np.arange(int(counts[i])) for i in images]
+    arrays = {"counts": counts, "images": images,
+              "boxes": np.concatenate([boxes[i, r] for i, r in zip(images, rows)]),
+              "scores": np.concatenate([scores[i, r] for i, r in zip(images, rows)]),
+              "cls": np.concatenate([cls[i, r] for i, r in zip(images, rows)])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.astype(np.float32))
+
+
 def bind_to_gpu_numa_node(index: int):
     """Restrict this rank to the CPU cores NVML reports as local to its GPU (before any pinned host
     buffer is allocated: first touch places the pages on that NUMA node).  With 8 ranks pushing
@@ -306,7 +342,6 @@ def main():
     if a.workload == "train":
         if a.impl == "reference":
             raise SystemExit("--workload train has no --impl reference arm (its CPU baseline is in the line itself)")
-        a.steps = min(a.steps, 30) if a.steps == 100 else a.steps
         run_train_workload(a)
         return
     rank = int(os.environ.get("RANK", "0"))
@@ -386,6 +421,8 @@ def main():
     ms_dev, _ = timed(step_dev, a.steps)
     launches = eng.launch_count - l0
     counts = out_dev[3].cpu().numpy()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, out_dev)
 
     # ---- end to end through the host-buffer C-ABI call (e2e) ---------------------------------
     # streaming use of the host API: step i is submitted (H2D on the copy stream, compute behind

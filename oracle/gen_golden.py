@@ -461,6 +461,40 @@ def letterbox_golden():
     print("g9_letterbox96.npz:", len(shapes), "images")
 
 
+def resize_cases():
+    """Yields (h0, w0, dw, dh, image) of the cv2 resize check: fixed shapes (the exact 2x downscale fast path,
+    up-scaling) and 25 random letterbox-style shapes, uint8 HWC noise images from one seeded generator."""
+    rng = np.random.default_rng(1)
+    shapes = [(480, 640, 416, 312), (640, 480, 312, 416), (100, 100, 416, 416), (832, 832, 416, 416), (37, 91, 416, 169)]
+    for _ in range(25):
+        h0, w0 = int(rng.integers(20, 700)), int(rng.integers(20, 700))
+        s = int(rng.choice([320, 416, 608]))
+        shapes.append((h0, w0, max(1, int(w0 / h0 * s)) if h0 > w0 else s, s if h0 >= w0 else max(1, int(h0 / w0 * s))))
+    for h0, w0, dw, dh in shapes:
+        yield h0, w0, dw, dh, rng.integers(0, 256, (h0, w0, 3), dtype=np.uint8)
+
+
+def resize_golden():
+    """g11: cv2.resize (INTER_LINEAR, the call inside ValTransforms) on the cases of resize_cases().  The outputs
+    are ~10 MB of noise, so each is stored as the SHA-256 of its bytes (bit-exact check) plus 256 values at seeded
+    positions (to show where a mismatch is); the input's SHA-256 pins the generated image."""
+    import hashlib
+    import cv2
+    out = {}
+    shapes = []
+    for i, (h0, w0, dw, dh, img) in enumerate(resize_cases()):
+        want = cv2.resize(img, (dw, dh))
+        idx = np.random.default_rng(i).choice(want.size, 256, replace=False)
+        shapes.append((h0, w0, dw, dh))
+        out[f"in_sha{i}"] = hashlib.sha256(img.tobytes()).hexdigest()
+        out[f"out_sha{i}"] = hashlib.sha256(want.tobytes()).hexdigest()
+        out[f"idx{i}"] = idx
+        out[f"vals{i}"] = want.reshape(-1)[idx]
+    np.savez_compressed(OUT / "g11_cv2resize.npz", cv2=cv2.__version__, numpy=np.__version__,
+                        shapes=np.array(shapes, dtype=np.int64), **out)
+    print("g11_cv2resize.npz:", len(shapes), "cases")
+
+
 def ema_golden():
     """g8: the REAL ModelEMA (utils/misc.py:67-86) over three updates of a model whose weights change between
     updates the way an optimizer would change them (deterministic perturbations)."""
@@ -495,6 +529,8 @@ if __name__ == "__main__":
         letterbox_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "ema":
         ema_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "resize":
+        resize_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "train":
         train_golden()
     else:

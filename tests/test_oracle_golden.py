@@ -198,16 +198,18 @@ def test_letterbox_transform_and_box_mapping_match_reference(golden):
         np.testing.assert_array_equal(got, g9[f"mapped{i}"])
 
 
-def test_cv2_resize_restatement_is_bit_exact():
-    """The restated OpenCV bilinear uint8 resize against the installed cv2 over random shapes (incl. the exact 2x
-    downscale fast path and up-scaling)."""
-    cv2 = pytest.importorskip("cv2")
-    rng = np.random.default_rng(1)
-    shapes = [(480, 640, 416, 312), (640, 480, 312, 416), (100, 100, 416, 416), (832, 832, 416, 416), (37, 91, 416, 169)]
-    for _ in range(25):
-        h0, w0 = int(rng.integers(20, 700)), int(rng.integers(20, 700))
-        s = int(rng.choice([320, 416, 608]))
-        shapes.append((h0, w0, max(1, int(w0 / h0 * s)) if h0 > w0 else s, s if h0 >= w0 else max(1, int(h0 / w0 * s))))
-    for h0, w0, dw, dh in shapes:
-        img = rng.integers(0, 256, (h0, w0, 3), dtype=np.uint8)
-        np.testing.assert_array_equal(O.cv2_resize_linear_u8(img, dw, dh), cv2.resize(img, (dw, dh)), err_msg=str((h0, w0, dw, dh)))
+def test_cv2_resize_restatement_is_bit_exact(golden):
+    """The restated OpenCV bilinear uint8 resize against cv2.resize over random shapes (incl. the exact 2x
+    downscale fast path and up-scaling), as recorded by oracle/gen_golden.py (golden g11: SHA-256 of every cv2
+    output plus 256 sampled values)."""
+    import hashlib
+    from oracle.gen_golden import resize_cases
+    g = golden("g11_cv2resize.npz")
+    cases = list(resize_cases())
+    assert [c[:4] for c in cases] == [tuple(s) for s in g["shapes"].tolist()]
+    for i, (h0, w0, dw, dh, img) in enumerate(cases):
+        assert hashlib.sha256(img.tobytes()).hexdigest() == str(g[f"in_sha{i}"]), f"input {i} is not the recorded one"
+        got = O.cv2_resize_linear_u8(img, dw, dh)
+        assert got.shape == (dh, dw, 3) and got.dtype == np.uint8, str((h0, w0, dw, dh))
+        np.testing.assert_array_equal(got.reshape(-1)[g[f"idx{i}"]], g[f"vals{i}"], err_msg=str((h0, w0, dw, dh)))
+        assert hashlib.sha256(got.tobytes()).hexdigest() == str(g[f"out_sha{i}"]), str((h0, w0, dw, dh))
