@@ -259,7 +259,11 @@ int  ynb_pwconv_tc(const float* in_dev, int32_t in_ld, int32_t in_off,
  * in_dev: NHWC view [batch][h][w][channels of in_ld], 16-byte aligned, channels % 4 == 0; dw_w_dev [9][channels]
  * tap-major, dw_b_dev [channels]; pw_w_dev [cout][channels], pw_b_dev [cout]; cout <= 128; out_dev / pass_dev
  * 16-byte aligned with out_ld, pass_ld multiples of 4 floats.
- * mode = YNB_GEMM_TC_3XTF32 | YNB_GEMM_TC_TF32.  Synchronous test hook (packs the weights on the host). */
+ * mode = YNB_GEMM_TC_3XTF32 | YNB_GEMM_TC_TF32 | YNB_GEMM_TC_BF16.  In bf16 mode in_dev, out_dev and pass_dev hold
+ * bf16 elements (in_ld, out_ld, channels multiples of 8; cout <= 240), the pointwise weights are rounded to bf16 and
+ * the depthwise output is rounded to bf16 before the GEMM; dw_w_dev, dw_b_dev, pw_b_dev stay float32.  Rows are
+ * written in whole 16-byte chunks there: with pass_dev, elements [2*cout, round_up(2*cout, 8)) of a row may be written.
+ * Synchronous test hook (packs the weights on the host). */
 int  ynb_dwpw_tc(const float* in_dev, int32_t in_ld, const float* dw_w_dev, const float* dw_b_dev, int32_t dw_act,
                  const float* pw_w_dev, const float* pw_b_dev, int32_t act,
                  float* out_dev, int32_t out_ld, const float* pass_dev, int32_t pass_ld,

@@ -111,7 +111,7 @@ def test_pwconv_strided_views(lib, G):
         assert float(out[:, 0::2].abs().max()) == 0.0
 
 
-@pytest.mark.parametrize("mode,tol", [(1, 3e-5), (2, 2e-2)])
+@pytest.mark.parametrize("mode,tol", [(1, 3e-5), (2, 2e-2), (3, 4e-3)])
 @pytest.mark.parametrize("batch,h,w,c,cout,dw_act,with_pass", [
     (2, 52, 52, 60, 58, 0, True),      # stage-2 stride-1 unit tail (58 channels stored with ld 60)
     (3, 26, 26, 116, 116, 0, True),    # stage 3: streamed weight chunks
@@ -123,9 +123,16 @@ def test_pwconv_strided_views(lib, G):
 ])
 def test_fused_dw_pw_unit_tail(lib, G, batch, h, w, c, cout, dw_act, with_pass, mode, tol):
     """dwpw_tc_kernel = depthwise 3x3 + bias (+act) -> pointwise + bias + act (+ cat/channel_shuffle with the
-    pass-through half) in one launch, against torch (backbone/shufflenetv2.py:57-63,70-76; models/yolo_nano.py:50-58)."""
+    pass-through half) in one launch, against torch (backbone/shufflenetv2.py:57-63,70-76; models/yolo_nano.py:50-58).
+    bf16 mode (3): in / out / pass are bf16 with channels and ld multiples of 8; the float64 reference rounds what the
+    kernel rounds (pointwise weights and the depthwise output, RNE), so the tolerance is the output's own rounding."""
+    bf = mode == 3
+    rnd = (lambda t: t.to(torch.bfloat16).double()) if bf else (lambda t: t)
+    al = 8 if bf else 4
+    up = lambda v: (v + al - 1) // al * al
     g = torch.Generator().manual_seed(h * 131 + c)
-    creal = min(c, 58) if c == 60 else c                      # physical pads (58 -> 60) carry zeros
+    creal = min(c, 58) if c == 60 else c                      # physical pads (58 -> 60, bf16: -> 64) carry zeros
+    c = up(c)
     x = torch.zeros(batch, h, w, c)
     x[..., :creal] = torch.randn(batch, h, w, creal, generator=g)
     dw_w = torch.zeros(c, 3, 3)
@@ -137,27 +144,29 @@ def test_fused_dw_pw_unit_tail(lib, G, batch, h, w, c, cout, dw_act, with_pass, 
     pw_b = torch.randn(cout, generator=g) * 0.3
     act = 2 if dw_act == 2 else 1
     f = {0: lambda t: t, 1: torch.relu, 2: lambda t: F.leaky_relu(t, 0.1)}
-    xn = x.permute(0, 3, 1, 2).double()
-    mid = f[dw_act](F.conv2d(xn, dw_w.double().unsqueeze(1), dw_b.double(), 1, 1, groups=c))
-    ref = f[act](F.conv2d(mid, pw_w.double()[:, :, None, None], pw_b.double())).permute(0, 2, 3, 1)
-    xd = x.to(G.DEV)
+    xn = rnd(x.permute(0, 3, 1, 2).double())
+    mid = rnd(f[dw_act](F.conv2d(xn, dw_w.double().unsqueeze(1), dw_b.double(), 1, 1, groups=c)))
+    ref = f[act](F.conv2d(mid, rnd(pw_w.double())[:, :, None, None], pw_b.double())).permute(0, 2, 3, 1)
+    et = torch.bfloat16 if bf else torch.float32
+    xd = x.to(G.DEV, et)
     dwp = dw_w.reshape(c, 9).t().contiguous().to(G.DEV)      # [9][C] tap-major
     dbd, pwd, pbd = dw_b.to(G.DEV), pw_w.contiguous().to(G.DEV), pw_b.to(G.DEV)
     if with_pass:
-        ld = 2 * cout + 4
-        pld = (cout + 3) // 4 * 4 + 4                                          # pass rows are read 16 bytes at a time
-        x1 = torch.randn(batch, h, w, pld, generator=g).to(G.DEV)
-        out = torch.full((batch, h, w, ld), float("nan"), device=G.DEV)
+        ld = up(2 * cout) + al
+        pld = up(cout) + al                                                    # pass rows are read 16 bytes at a time
+        x1 = torch.randn(batch, h, w, pld, generator=g).to(G.DEV, et)
+        out = torch.full((batch, h, w, ld), float("nan"), device=G.DEV, dtype=et)
         rc = lib.ynb_dwpw_tc(G.ptr(xd), c, G.ptr(dwp), G.ptr(dbd), dw_act, G.ptr(pwd), G.ptr(pbd), act, G.ptr(out), ld,
                              G.ptr(x1), pld, batch, h, w, c, cout, mode, G.stream())
         assert rc == 0, lib.ynb_last_error(None)
         torch.cuda.synchronize()
         assert torch.equal(out[..., 0:2 * cout:2], x1[..., :cout])           # pass-through half, bit for bit
         torch.testing.assert_close(out[..., 1:2 * cout:2].double().cpu(), ref, rtol=tol, atol=tol)
-        assert bool(torch.isnan(out[..., 2 * cout:]).all())                  # nothing written past the unit's channels
+        # nothing written past the unit's channels (bf16: past its last 16-byte chunk, round_up(2 * cout, 8))
+        assert bool(torch.isnan(out[..., up(2 * cout):]).all())
     else:
-        ld = (cout + 3) // 4 * 4 + 4
-        out = torch.full((batch, h, w, ld), float("nan"), device=G.DEV)
+        ld = up(cout) + al
+        out = torch.full((batch, h, w, ld), float("nan"), device=G.DEV, dtype=et)
         rc = lib.ynb_dwpw_tc(G.ptr(xd), c, G.ptr(dwp), G.ptr(dbd), dw_act, G.ptr(pwd), G.ptr(pbd), act, G.ptr(out), ld,
                              None, 0, batch, h, w, c, cout, mode, G.stream())
         assert rc == 0, lib.ynb_last_error(None)

@@ -1275,11 +1275,12 @@ YNB_EXPORT int ynb_commit_weights(ynb_engine* e) {
     int rc = pack_conv(e, (int)i);
     if (rc) return rc;
   }
-  if (e->cfg.gemm_mode != YNB_GEMM_FP32_FFMA)
-    for (int si = 0; si < 3; ++si) {
-      int rc = pack_cat(e, si);
-      if (rc) return rc;
-    }
+  // The merged stride-2 weights depend only on the storage type, not on the GEMM mode: pack them in FFMA mode too,
+  // or a later ynb_set_gemm_mode to a tensor-core mode would run the stride-2 units on the previous weights.
+  for (int si = 0; si < 3; ++si) {
+    int rc = pack_cat(e, si);
+    if (rc) return rc;
+  }
   e->committed = true;
   return YNB_OK;
 }

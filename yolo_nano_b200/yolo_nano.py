@@ -231,11 +231,16 @@ class YOLONano(nn.Module):
         return out
 
     def _weight_tensors(self):
-        """The 469 (154 after fuse_conv_bn) tensors the engine weights are derived from, cached per module
-        structure (fuse_conv_bn replaces modules: `_modules` ids change and the list is rebuilt)."""
-        key = tuple(id(m) for m in self.modules())
-        if self._wt_cache is None or self._wt_cache[0] != key:
-            object.__setattr__(self, "_wt_cache", (key, list(self.state_dict(keep_vars=True).values())))
+        """The 469 (154 after fuse_conv_bn) tensors the engine weights are derived from.  The list is cached
+        together with every (`_modules` / `_parameters` / `_buffers` dict, key, object) slot of the module tree
+        and rebuilt as soon as one slot holds another object: fuse_conv_bn replaces modules, and
+        `load_state_dict(assign=True)` and dtype / device conversions put new tensor objects in place, whose
+        changes the fingerprint of the old objects would never see.  The check is identity only (~30 us)."""
+        c = self._wt_cache
+        if c is None or not all(d.get(k) is v for d, k, v in c[0]):
+            slots = [(d, k, v) for m in self.modules() for d in (m._modules, m._parameters, m._buffers)
+                     for k, v in d.items() if v is not None]
+            object.__setattr__(self, "_wt_cache", (slots, list(self.state_dict(keep_vars=True).values())))
         return self._wt_cache[1]
 
     def _weights_fingerprint(self):
