@@ -231,6 +231,40 @@ int  ynb_preprocess_letterbox_u8(ynb_engine* e, const uint8_t* src_dev, const yn
 int  ynb_map_boxes(float* boxes_dev, const int32_t* counts_dev, const double* maps_dev, int32_t batch,
                    int64_t n_per_image, void* stream);
 
+/* VOC mAP on the device (evaluator/vocapi_evaluator.py: write_voc_results_file + voc_eval + voc_ap, ssd.pytorch
+ * lineage: overlaps without the +1 pixel, ap = -1 for a class without detection lines).
+ *
+ * ynb_voc_append turns the kept rows of a batch (after ynb_map_boxes: pixel boxes [batch][n_per_image][4], scores
+ * [batch][n_per_image], cls [batch][n_per_image], counts [batch]) into det-file lines, one int32 row each:
+ *     rows_dev[slot] = {image_base + b, class, milli, x1, y1, x2, y2}
+ * milli is the integer of '{:.3f}' of the score and xk the integer of '{:.1f}' of (box_k + 1), the +1 added in
+ * float32; both round half-even on the exact binary value like Python's formatting, so milli / 1000.0 and
+ * xk / 10.0 are the doubles voc_eval parses back.  A '-0.0' field is stored as INT32_MIN.  Slots follow file order
+ * (image, then kept row): state_dev[0] (int64, zeroed by the caller before the first batch) holds the rows
+ * appended so far and is advanced on the device; rows at or past `capacity` are counted but not written.
+ * state_dev[1] counts rejected values (class out of range, score outside [0, 1], non-finite or |box + 1| >= 2^27);
+ * their rows are written clamped, and the caller must not evaluate them. */
+int  ynb_voc_append(const float* boxes_dev, const float* scores_dev, const int32_t* cls_dev,
+                    const int32_t* counts_dev, int32_t batch, int64_t n_per_image, int32_t image_base,
+                    int32_t num_classes, int32_t* rows_dev, int64_t capacity, int64_t* state_dev, void* stream);
+
+/* voc_eval of every class over rows_dev[0, n_rows) (the caller reads n_rows from state_dev[0] and checks it
+ * against the capacity).  Ground truth in voc_eval's coordinates, bucketed by (image, class) in annotation order:
+ * GT g has gt_boxes_dev[g][4] (float64 x1, y1, x2, y2) and gt_difficult_dev[g]; bucket (i, c) is
+ * [gt_start_dev[i * num_classes + c], gt_start_dev[i * num_classes + c + 1]), gt_start_dev has
+ * num_images * num_classes + 1 entries.  Detections are ordered by score descending, ties by file order; a
+ * detection is TP when its best overlap (> ovthresh, strict) hits a non-difficult GT that no earlier detection
+ * claimed, ignored on a difficult one.  Outputs: ap_dev [num_classes] float64 (VOC07 11-point when use_07_metric,
+ * else the area under the precision envelope; -1 for a class without rows), npos_dev [num_classes] (non-difficult
+ * GT per class); optional (NULL to skip) order_dev [n_rows] = arena row of each sorted position and flags_dev
+ * [n_rows] = 1 TP, 2 FP, 0 ignored per sorted position.  Deterministic. */
+int64_t ynb_voc_eval_workspace_bytes(int64_t n_rows, int32_t num_classes, int64_t n_gt);
+int  ynb_voc_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num_classes, int32_t num_images,
+                  const double* gt_boxes_dev, const uint8_t* gt_difficult_dev, const int32_t* gt_start_dev,
+                  int64_t n_gt, double ovthresh, int32_t use_07_metric, double* ap_dev, int32_t* npos_dev,
+                  int32_t* order_dev, int8_t* flags_dev, void* workspace_dev, int64_t workspace_bytes,
+                  void* stream);
+
 /* Pointwise 1x1 conv = GEMM over pixels, + bias + activation, fp32 FFMA variant
  * (backbone/shufflenetv2.py:46,54,60; utils/modules.py:11 with k=1).
  * w_dev is [cout][cin] row-major, b_dev [cout].

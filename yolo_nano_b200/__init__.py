@@ -12,6 +12,7 @@ from .engine import Engine, EngineError  # noqa: F401
 from .tta import TestTimeAugmentation, resize_bilinear  # noqa: F401
 from .ema import ModelEMA  # noqa: F401
 from . import evalfmt  # noqa: F401
+from .voc_eval import VOCDetections  # noqa: F401
 
 # anchors of the reference (data/config.py:11-17): constructor inputs, data not code
 MULTI_ANCHOR_SIZE = [[30.65, 39.12], [50.3, 102.62], [94.98, 64.55],

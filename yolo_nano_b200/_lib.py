@@ -85,6 +85,10 @@ SIGNATURES = {
     "ynb_preprocess_u8": (C.c_int, [_p, _p, _p, _i32, _p, _p]),
     "ynb_preprocess_letterbox_u8": (C.c_int, [_p, _p, _p, _i32, _p, _p]),
     "ynb_map_boxes": (C.c_int, [_p, _p, _p, _i32, _i64, _p]),
+    "ynb_voc_append": (C.c_int, [_p, _p, _p, _p, _i32, _i64, _i32, _i32, _p, _i64, _p, _p]),
+    "ynb_voc_eval_workspace_bytes": (_i64, [_i64, _i32, _i64]),
+    "ynb_voc_eval": (C.c_int, [_p, _i64, _i32, _i32, _p, _p, _p, _i64, C.c_double, _i32, _p, _p, _p, _p, _p, _i64,
+                               _p]),
     "ynb_submit_host_u8": (C.c_int, [_p, _i32, _p, _p, _i32, _p, _p, _p, _p, _p]),
     "ynb_nms_grid_workspace_bytes": (_i64, [_i32, _i32]),
     "ynb_nms_grid": (C.c_int, [_p, _p, _p, _i32, _i32, _i32, _f, _f, _i32,

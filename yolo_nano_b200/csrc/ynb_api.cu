@@ -26,6 +26,7 @@
 #include "kernels_basic.cuh"
 #include "train_ops.cuh"
 #include "wgrad_tc.cuh"
+#include "voc_eval.cuh"
 #include "topology.h"
 
 #define YNB_EXPORT extern "C" __attribute__((visibility("default")))
@@ -1489,6 +1490,49 @@ YNB_EXPORT int ynb_map_boxes(float* boxes_dev, const int32_t* counts_dev, const 
     return fail(nullptr, YNB_ERR_INVALID, "ynb_map_boxes: bad arguments");
   cudaError_t r = launch_map_boxes(boxes_dev, counts_dev, maps_dev, batch, n_per_image, (cudaStream_t)stream);
   if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("map_boxes: ") + cudaGetErrorString(r));
+  return YNB_OK;
+}
+
+// Sorted positions and GT claims are int32 (claims start at 0x7f7f7f7f): the arena stays below that.
+constexpr int64_t kVocMaxRows = 0x7f000000;
+constexpr int32_t kVocMaxClasses = 4096;
+
+YNB_EXPORT int ynb_voc_append(const float* boxes_dev, const float* scores_dev, const int32_t* cls_dev,
+                              const int32_t* counts_dev, int32_t batch, int64_t n_per_image, int32_t image_base,
+                              int32_t num_classes, int32_t* rows_dev, int64_t capacity, int64_t* state_dev,
+                              void* stream) {
+  if (!boxes_dev || !scores_dev || !cls_dev || !counts_dev || !rows_dev || !state_dev || batch <= 0 ||
+      n_per_image <= 0 || image_base < 0 || (int64_t)image_base + batch > INT32_MAX || num_classes < 1 ||
+      num_classes > kVocMaxClasses || capacity < 0 || capacity > kVocMaxRows)
+    return fail(nullptr, YNB_ERR_INVALID, "ynb_voc_append: bad arguments");
+  cudaError_t r = ynb::voc::launch_voc_append(boxes_dev, scores_dev, cls_dev, counts_dev, batch, n_per_image,
+                                              image_base, num_classes, rows_dev, capacity,
+                                              reinterpret_cast<long long*>(state_dev), (cudaStream_t)stream);
+  if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("voc_append: ") + cudaGetErrorString(r));
+  return YNB_OK;
+}
+
+YNB_EXPORT int64_t ynb_voc_eval_workspace_bytes(int64_t n_rows, int32_t num_classes, int64_t n_gt) {
+  if (n_rows < 0 || n_rows > kVocMaxRows || num_classes < 1 || num_classes > kVocMaxClasses || n_gt < 0) return -1;
+  return ynb::voc::eval_workspace(nullptr, n_rows, num_classes, n_gt, nullptr);
+}
+
+YNB_EXPORT int ynb_voc_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num_classes, int32_t num_images,
+                            const double* gt_boxes_dev, const uint8_t* gt_difficult_dev, const int32_t* gt_start_dev,
+                            int64_t n_gt, double ovthresh, int32_t use_07_metric, double* ap_dev, int32_t* npos_dev,
+                            int32_t* order_dev, int8_t* flags_dev, void* workspace_dev, int64_t workspace_bytes,
+                            void* stream) {
+  const int64_t need = ynb_voc_eval_workspace_bytes(n_rows, num_classes, n_gt);
+  if (need < 0 || num_images < 0 || (int64_t)num_images * num_classes > INT32_MAX || n_gt > INT32_MAX ||
+      (n_rows > 0 && !rows_dev) || (n_gt > 0 && (!gt_boxes_dev || !gt_difficult_dev)) || !gt_start_dev ||
+      !ap_dev || !npos_dev || !workspace_dev || workspace_bytes < need)
+    return fail(nullptr, YNB_ERR_INVALID, "ynb_voc_eval: bad arguments / workspace too small");
+  ynb::voc::EvalWorkspace w;
+  ynb::voc::eval_workspace(workspace_dev, n_rows, num_classes, n_gt, &w);
+  cudaError_t r = ynb::voc::launch_voc_eval(rows_dev, n_rows, num_classes, num_images, gt_boxes_dev,
+                                            gt_difficult_dev, gt_start_dev, n_gt, ovthresh, use_07_metric ? 1 : 0,
+                                            ap_dev, npos_dev, order_dev, flags_dev, w, (cudaStream_t)stream);
+  if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("voc_eval: ") + cudaGetErrorString(r));
   return YNB_OK;
 }
 

@@ -305,12 +305,13 @@ class Engine:
         for i, im in enumerate(images):
             o = int(descs[i]["offset"])
             pk[o:o + im.size] = np.ascontiguousarray(im).reshape(-1)
+        # pinned staging + non_blocking: the host does not wait for the copies (a batch loop stays asynchronous)
         src = packed.to(self.device, non_blocking=True)
-        d_desc = torch.from_numpy(descs.view(np.uint8).reshape(-1)).to(self.device)
+        d_desc = torch.from_numpy(descs.view(np.uint8).reshape(-1)).pin_memory().to(self.device, non_blocking=True)
         x = torch.empty((len(images), 3, s, s), dtype=torch.float32, device=self.device)
         self._check(self.lib.ynb_preprocess_letterbox_u8(self._h, _ptr(src), _ptr(d_desc), len(images), _ptr(x),
                                                          _stream_ptr(self.device)), "ynb_preprocess_letterbox_u8")
-        return x, torch.from_numpy(maps).to(self.device)
+        return x, torch.from_numpy(maps).pin_memory().to(self.device, non_blocking=True)
 
     def map_boxes(self, boxes: torch.Tensor, counts: torch.Tensor, maps: torch.Tensor):
         """In place: boxes [B,N,4] (normalised, NMS output) -> original image pixels, rows [0, counts[b])

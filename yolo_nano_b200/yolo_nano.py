@@ -365,6 +365,38 @@ class YOLONano(nn.Module):
                  np.array(sh[b, :int(counts_h[b])], dtype=np.float32, copy=True),
                  ch[b, :int(counts_h[b])].astype(np.int64)) for b in range(nb)]
 
+    def evaluate_voc(self, images, gt, batch_size: int = 64, use_07_metric: bool = True, ovthresh: float = 0.5,
+                     capacity: Optional[int] = None):
+        """`VOCAPIEvaluator.evaluate` + `do_python_eval` (evaluator/vocapi_evaluator.py) on the device: `images` is an
+        iterable of ORIGINAL uint8 BGR images, `gt` one (boxes [G,4], labels [G], difficult [G]) per image in
+        voc_eval's coordinates.  Per batch: ValTransforms, detection, the inverse box mapping and the det-file lines
+        stay on the device; the host waits once, for the APs.  Returns (aps float64 [C], mAP).  `capacity` bounds
+        the detection lines (default: every anchor box of every image, which cannot overflow)."""
+        from .voc_eval import VOCDetections
+        if batch_size < 1:
+            raise ValueError("batch_size must be positive")
+        eng = self.engine(batch_size)
+        if capacity is None:
+            capacity = len(gt) * eng.num_boxes
+        dets = VOCDetections(eng.device, self.num_classes, capacity)
+        batch = []
+
+        def run(batch):
+            eng = self.engine(len(batch))
+            x, maps = eng.preprocess_images(batch)
+            boxes, scores, cls, counts = eng.forward_detect(x)
+            eng.map_boxes(boxes, counts, maps)
+            dets.add(boxes, scores, cls, counts)
+
+        for im in images:
+            batch.append(im)
+            if len(batch) == batch_size:
+                run(batch)
+                batch = []
+        if batch:
+            run(batch)
+        return dets.evaluate(gt, ovthresh=ovthresh, use_07_metric=use_07_metric)
+
     def forward(self, x, target=None):
         if self.trainable:
             # training branch (models/yolo_nano.py:333-358).  The returned losses are plain device scalars WITHOUT a
