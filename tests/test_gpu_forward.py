@@ -1,5 +1,6 @@
 """End-to-end parity of the engine and the drop-in module on a real B200."""
 import contextlib
+import ctypes as C
 import io
 
 import numpy as np
@@ -228,19 +229,37 @@ def test_g3_416_against_reference(G, golden):
 
 
 @pytest.mark.parametrize("classes,size", [(80, 128), (20, 160)])
-def test_fused_decode_epilogue_equals_decode_kernel(G, classes, size, monkeypatch):
+def test_fused_decode_epilogue_equals_decode_kernel(lib, G, classes, size):
     """head_det_*.4 with the decode in the GEMM epilogue (no raw map in HBM) against the same
     conv followed by decode_level_kernel: identical raw sums feed identical arithmetic, so
-    boxes and scores are bit-equal; classes may differ only where two products round equal."""
+    boxes and scores are bit-equal; classes may differ only where two products round equal.
+    The reference is the engine's raw tail (planned with the same merged accumulator as the
+    fused tail), laid out NHWC again and decoded level by level by ynb_decode_level."""
     sd = W.calibrated(classes, seed=5)
-    x = W.synthetic_input(3, size, 5).to(G.DEV)
-    eng_f = G.make_engine(sd, size, classes, "3xtf32")
-    bf, sf, cf = [t.cpu().numpy() for t in eng_f.forward_decode(x)]
-    eng_f.close()
-    monkeypatch.setenv("YNB_NO_FUSED_DECODE", "1")
-    eng_u = G.make_engine(sd, size, classes, "3xtf32")
-    bu, su, cu = [t.cpu().numpy() for t in eng_u.forward_decode(x)]
-    eng_u.close()
+    batch = 3
+    x = W.synthetic_input(batch, size, 5).to(G.DEV)
+    eng = G.make_engine(sd, size, classes, "3xtf32")
+    bf, sf, cf = [t.cpu().numpy() for t in eng.forward_decode(x)]
+    raw = eng.forward_raw(x)
+    eng.close()
+    ch = 3 * (1 + classes + 4)
+    ld = (ch + 3) // 4 * 4
+    n = sum(3 * (size // s) ** 2 for s in (8, 16, 32))
+    boxes = torch.zeros(batch, n, 4, device=G.DEV)
+    scores = torch.zeros(batch, n, device=G.DEV)
+    cl = torch.zeros(batch, n, device=G.DEV, dtype=torch.int32)
+    anchors = np.array(W.anchors_for(classes), dtype=np.float32).reshape(3, 6)
+    off = 0
+    for lvl, p in enumerate(raw):
+        gsz = p.shape[2]
+        nhwc = torch.zeros(batch, gsz * gsz, ld, device=G.DEV)
+        nhwc[..., :ch] = p.permute(0, 2, 3, 1).reshape(batch, gsz * gsz, ch)
+        a = (C.c_float * 6)(*anchors[lvl].tolist())
+        rc = lib.ynb_decode_level(G.ptr(nhwc), ld, G.ptr(boxes), G.ptr(scores), G.ptr(cl), batch, gsz, 8 << lvl, size,
+                                  a, 3, classes, n, off, G.stream())
+        assert rc == 0, lib.ynb_last_error(None)
+        off += gsz * gsz * 3
+    bu, su, cu = boxes.cpu().numpy(), scores.cpu().numpy(), cl.cpu().numpy()
     np.testing.assert_array_equal(bf, bu)
     np.testing.assert_array_equal(sf, su)
     assert (cf != cu).mean() < 1e-4

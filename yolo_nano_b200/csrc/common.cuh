@@ -3,7 +3,6 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <limits.h>
 #include <stdlib.h>
 
 #include "yolonano_b200.h"
@@ -25,17 +24,6 @@ __device__ __forceinline__ float apply_act(float v, int act) {
 // 2 instructions instead of expf's 7.
 __device__ __forceinline__ float softmax_exp(float d) { return __expf(d); }
 __device__ __forceinline__ float class_score(float sum, float obj) { return __fmul_rn(__fdiv_rn(1.0f, sum), obj); }
-
-// A view of an NHWC activation: `ld` floats between pixels, channels [off, off+c) used.
-// Stage-2 tensors (116 = 2 x 58 channels) are stored as [58 | 2 zero pads | 58 | 2 zero
-// pads] so that both halves start 16-byte aligned (TMA / float4 need it): logical
-// channel j lives in slot j + (j >= gap_at ? gap : 0).
-struct ChanMap {
-  int gap_at;   // INT_MAX when the layout is dense
-  int gap;
-  __host__ __device__ __forceinline__ int slot(int j) const { return j + (j >= gap_at ? gap : 0); }
-};
-__host__ __device__ inline ChanMap dense_map() { return ChanMap{INT_MAX, 0}; }
 
 // ---- activation storage type: float32 (parity / tf32 modes) or bfloat16 (YNB_GEMM_TC_BF16) ---------------
 // Arithmetic is always fp32 (depthwise taps, bias, activation, accumulators); only what sits in HBM between

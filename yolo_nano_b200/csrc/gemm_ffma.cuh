@@ -27,7 +27,6 @@ struct GemmParams {
   // output
   float* out;
   int out_ld, out_off, out_step;
-  ChanMap omap;
   int64_t M;
   int N, Ktot;       // Ktot multiple of 4
   int act;
@@ -173,11 +172,11 @@ gemm_ffma_kernel(GemmParams p) {
     int n = n0 + tx + 16 * j;
     if (n >= p.N) continue;
     float bj = __ldg(p.bias + n);
-    int slot = p.omap.slot(p.out_off + n * p.out_step);
+    int col = p.out_off + n * p.out_step;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       int64_t m = m0 + ty * 8 + i;
-      if (m < p.M) p.out[m * p.out_ld + slot] = apply_act(acc[i][j] + bj, p.act);
+      if (m < p.M) p.out[m * p.out_ld + col] = apply_act(acc[i][j] + bj, p.act);
     }
   }
 }

@@ -53,7 +53,6 @@ constexpr int kTcBK = 32;                       // floats per K chunk = 128 byte
 constexpr int kTcAStageBytes = kTcBM * 128;     // 16 KB
 constexpr int kTcMaxStages = 8;
 constexpr int kTcSmemBudget = 232448;                   // 227 KB opt-in maximum (layout totals include the alignment slack)
-constexpr int kTcMaxMain = 4;
 
 struct TcGemmParams {
   int num_steps;          // K chunks per tile (pointwise: ceil(K/32); 3x3: 9 * C/32)
@@ -68,8 +67,7 @@ struct TcGemmParams {
   int64_t num_tiles;
   int H, W, TH, TW, tiles_x, tiles_y;   // 3x3 spatial tiling
   int N, Npad;
-  int nmain;              // main accumulators (round-robin over K steps), 1..4
-  int nacc;               // accumulators per stage = nmain + (parity mode ? 1 correction : 0)
+  int nacc;               // accumulators per stage: 2 (main + correction) in parity mode unless merged, else 1
   int merge_corr;         // parity mode, shallow K: corrections go into the single main accumulator (nacc = 1)
   int ksub;               // pointwise: valid 8-float K sub-steps = ceil(K / 8) (sub-steps made only of zero padding are
                           // not issued: K = 116 needs 15 of 16, K = 232 29 of 32, K = 24 3 of 4); 0 = all
@@ -78,7 +76,7 @@ struct TcGemmParams {
   int a2_step;            // pointwise, > 0: K steps [a2_step, num_steps) read a SECOND activation tensor (tmAlo) — the
                           // two branches of a stride-2 ShuffleNetV2 unit concatenated along K against block-diagonal,
                           // row-interleaved weights: torch.cat + channel_shuffle as one plain GEMM output
-  int stack_b;            // parity mode, nmain = 1, 2*Npad <= 256: a_hi x [b_hi; b_lo] as ONE MMA of N = 2*Npad
+  int stack_b;            // parity mode, 2*Npad <= 256: a_hi x [b_hi; b_lo] as ONE MMA of N = 2*Npad
                           // into [main | corr] (the planes are adjacent in smem and in TMEM): 2 MMAs per
                           // K-step instead of 3, a_hi and b_hi are fetched once less
   int acc_stages;         // TMEM accumulator stages (2 = epilogue overlaps the next tile's MMAs)
@@ -87,12 +85,11 @@ struct TcGemmParams {
   // epilogue
   float* out;
   int out_ld, out_off, out_step;
-  ChanMap omap;
   const float* bias;
   int act;
   // Stride-1 ShuffleNetV2 unit: this GEMM is branch2's last conv; `pass` points at the
   // pass-through half x1 (same pixels, `N` channels).  The epilogue then writes whole
-  // interleaved rows out[slot(2i)] = x1[i], out[slot(2i+1)] = branch2[i]  — torch.cat +
+  // interleaved rows out[2i] = x1[i], out[2i+1] = branch2[i]  — torch.cat +
   // channel_shuffle (backbone/shufflenetv2.py:70-76, 14-28) as one coalesced store.
   const float* pass;
   int pass_ld;
@@ -317,7 +314,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         ptx::tc_fence_after_sync();
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * acc_cols);
         // correction accumulator (the main one itself when merged: its first MMA initialises it)
-        const uint32_t c_tmem = p.merge_corr ? d_tmem : d_tmem + (uint32_t)(p.nmain * p.Npad);
+        const uint32_t c_tmem = p.merge_corr ? d_tmem : d_tmem + (uint32_t)p.Npad;
         int t = 0;                                                       // K-step counter of the tile
         for (int st = 0; st < p.num_steps; ++st) {
           ok = ptx::mbar_wait(splitters_on ? &ready[s] : &full[s], ph, p.err_flag, 4);
@@ -352,13 +349,11 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const uint32_t ko = k * 32;   // 8 tf32 = 32 bytes inside the 128-byte swizzled row
               const uint64_t da = ptx::make_sw128_kmajor_desc(a_hi + ko);
               const uint64_t db = ptx::make_sw128_kmajor_desc(b_hi + ko);
-              const int slot = t % p.nmain;
               if (split) {
                 ptx::mma_tf32_ss(c_tmem, ptx::make_sw128_kmajor_desc(a_lo + ko), db, idesc, t != 0);
                 ptx::mma_tf32_ss(c_tmem, da, ptx::make_sw128_kmajor_desc(b_lo + ko), idesc, 1);
               }
-              ptx::mma_tf32_ss(d_tmem + (uint32_t)(slot * p.Npad), da, db, idesc,
-                               (split && p.merge_corr) ? 1 : (t >= p.nmain));
+              ptx::mma_tf32_ss(d_tmem, da, db, idesc, (split && p.merge_corr) ? 1 : (t != 0));
             }
           }
           YNB_TRACE(3, tile, st);
@@ -410,7 +405,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int group = warp >> 2;
     const int q = warp & 3;                         // TMEM lane quarter this warp may read
     const int row = q * 32 + lane;                  // tile row owned by this thread
-    const bool vec = p.out_step == 1 && p.omap.gap == 0;
+    const bool vec = p.out_step == 1;
     const float slope = p.act == YNB_ACT_RELU ? 0.0f : (p.act == YNB_ACT_LEAKY ? 0.1f : 1.0f);
     uint8_t* sbox = smem + lay.stg_off + warp * 4096;          // this warp's [32 rows x 128 B] swizzled box
     const int sw = lane & 7;                                    // swizzle phase of this thread's row
@@ -489,14 +484,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         auto ld16 = [&](int c0, float (&v)[16]) {          // 16 raw columns: accumulator sum(s), no bias yet
           uint32_t r[16];
           ptx::tmem_ld_32x16(t_base + c0, r);
-          if (p.nacc > 1) {
-            for (int a2 = 1; a2 < p.nacc; ++a2) {
-              uint32_t r2[16];
-              ptx::tmem_ld_32x16(t_base + (uint32_t)(a2 * p.Npad) + c0, r2);
-              ptx::tmem_ld_wait();
+          if (p.nacc == 2) {
+            uint32_t r2[16];
+            ptx::tmem_ld_32x16(t_base + (uint32_t)p.Npad + c0, r2);
+            ptx::tmem_ld_wait();
 #pragma unroll
-              for (int jj = 0; jj < 16; ++jj) r[jj] = __float_as_uint(__uint_as_float(r[jj]) + __uint_as_float(r2[jj]));
-            }
+            for (int jj = 0; jj < 16; ++jj) r[jj] = __float_as_uint(__uint_as_float(r[jj]) + __uint_as_float(r2[jj]));
           }
           ptx::tmem_ld_wait();
 #pragma unroll
@@ -583,7 +576,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (lane == 0 && q == 0) YNB_TRACE(5, tile, group);
         continue;
       }
-      // 16 columns: sum of the accumulators (main_0 + main_1 + ... + correction) + bias, activation
+      // 16 columns: sum of the accumulators (main + correction) + bias, activation
       // (branch-free: act(x) = max(x, slope*x), slope 1 / 0 / 0.1 = identity / ReLU / LeakyReLU(0.1)),
       // written as chunks jc..jc+3 of this thread's swizzled 128-byte line
       // The previous TMA store of this warp must have finished READING the staging box before it is rewritten: waited
@@ -597,20 +590,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       auto drain16 = [&](int c0, int jc) {
         uint32_t r[16];
         ptx::tmem_ld_32x16(t_base + c0, r);
-        if (p.nacc == 2) {            // main + correction (the common case): both loads, one wait
+        if (p.nacc == 2) {            // main + correction: both loads, one wait
           uint32_t r2[16];
           ptx::tmem_ld_32x16(t_base + (uint32_t)p.Npad + c0, r2);
           ptx::tmem_ld_wait();
 #pragma unroll
           for (int j = 0; j < 16; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(r2[j]));
-        } else if (p.nacc > 2) {
-          for (int a = 1; a < p.nacc; ++a) {
-            uint32_t r2[16];
-            ptx::tmem_ld_32x16(t_base + (uint32_t)(a * p.Npad) + c0, r2);
-            ptx::tmem_ld_wait();
-#pragma unroll
-            for (int j = 0; j < 16; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(r2[j]));
-          }
         } else {
           ptx::tmem_ld_wait();
         }
@@ -675,9 +660,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int i = c0 + lane;                                // output channel of this lane
         const bool col_ok = i < p.N;
         if (kPass) {
-          // out[slot(2i)] = x1[i] (pass-through), out[slot(2i+1)] = branch2[i]: 256-byte row segments
+          // out[2i] = x1[i] (pass-through), out[2i+1] = branch2[i]: 256-byte row segments
           const int nrow = col_ok ? (int)min((int64_t)32, p.M - m_base) : 0;   // rows this lane stores
-          float* o = p.out + m_base * p.out_ld + p.omap.slot(2 * (col_ok ? i : 0));
+          float* o = p.out + m_base * p.out_ld + 2 * (col_ok ? i : 0);
 #pragma unroll
           for (int r = 0; r < 16; ++r, o += p.out_ld)
             if (r < nrow) *reinterpret_cast<float2*>(o) = make_float2(xa[r], staged(r, lane));
@@ -687,7 +672,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (r < nrow) *reinterpret_cast<float2*>(o) = make_float2(xb[r - 16], staged(r, lane));
           if (c0 + 32 < col_end) fetch_x1(c0 + 32, 16, xb);
         } else {
-          const int col = vec ? p.out_off + i : p.omap.slot(p.out_off + (col_ok ? i : 0) * p.out_step);
+          const int col = p.out_off + (vec ? i : (col_ok ? i : 0) * p.out_step);
           if (!p.is3x3) {
             const int nrow = col_ok ? (int)min((int64_t)32, p.M - m_base) : 0;
             if (p.out_bf16) {
@@ -850,51 +835,23 @@ struct TcGemmLaunch {
   int dec_classes = 0;    // 80 | 20: fused decode epilogue (p.dec valid); 0: ordinary epilogue
 };
 
-// TMEM plan (512 columns).  Parity mode: one correction accumulator plus `nmain` main
-// accumulators — more of them the deeper K is (truncation bias grows with the number of
-// accumulation steps).  Two accumulator stages (epilogue of tile i overlaps the MMAs of tile
-// i+1) whenever they fit; a shallow K gives up an extra main accumulator for that overlap, a
-// deep K (3x3 convs: 108 steps, K=464 laterals) keeps the accumulators and runs single-stage.
+// TMEM plan (512 columns).  Parity mode: one main accumulator plus one correction accumulator.
+// Measured (B200, calibrated weights, 128^2 and 416^2): with the round-to-nearest split and the
+// corrections in their own accumulator, ONE main accumulator gives the same end-to-end error as
+// four round-robin ones (box error 0.024 vs 0.025 px, identical keep sets) — and it lets the hi/lo
+// weight planes be stacked into one MMA and the 3x3 convs double-buffer their accumulators: 3x3
+// convs 2x faster.  Two accumulator stages (epilogue of tile i overlaps the MMAs of tile i+1)
+// whenever they fit.
 inline void tc_plan_tmem(TcGemmParams& p, bool allow_merge = false) {
   const bool split = p.mode == YNB_GEMM_TC_3XTF32;
-  p.merge_corr = 0;
-  static const bool merge_all = getenv("YNB_TC_MERGE_ALL") != nullptr;     // experiment: one accumulator everywhere
-  if (split && ((allow_merge && p.num_steps * (kTcBK / 8) <= 16) || merge_all) && 2 * p.Npad <= 512) {
-    // <= 16 K steps (48 accumulations): the one-sided truncation of a single accumulator stays
-    // below 3e-6 relative — buys two accumulator stages for N = 256 (fused decode heads)
-    p.merge_corr = 1;
-    p.stack_b = 0;
-    p.nmain = 1; p.nacc = 1; p.acc_stages = 2;
-    p.tmem_cols = 32;
-    while ((int)p.tmem_cols < 2 * p.Npad) p.tmem_cols <<= 1;
-    return;
-  }
-  const int corr = split ? 1 : 0;
-  int want = 1;
-  if (split) {
-    const int ksteps = p.num_steps * (kTcBK / 8);
-    want = ksteps >= 64 ? 4 : (ksteps >= 24 ? 3 : (ksteps >= 12 ? 2 : 1));
-    // Measured (B200, calibrated weights, 128^2 and 416^2): with the round-to-nearest split and the
-    // corrections in their own accumulator, ONE main accumulator gives the same end-to-end error as
-    // four (box error 0.024 vs 0.025 px, identical keep sets) — and it lets the hi/lo weight planes be
-    // stacked into one MMA and the 3x3 convs double-buffer their accumulators: 3x3 convs 2x faster.
-    // YNB_TC_NMAIN_MAX=4 restores the round-robin main accumulators for comparison.
-    static const int nmain_cap = getenv("YNB_TC_NMAIN_MAX") ? atoi(getenv("YNB_TC_NMAIN_MAX")) : 1;
-    if (want > nmain_cap) want = nmain_cap;
-  }
-  p.nmain = want;
-  while (p.nmain > 1 && (p.nmain + corr) * p.Npad > 512) p.nmain--;
-  p.nacc = p.nmain + corr;
+  // <= 16 K steps (48 accumulations): the one-sided truncation of a single accumulator stays
+  // below 3e-6 relative — buys two accumulator stages for N = 256 (fused decode heads)
+  p.merge_corr = (split && allow_merge && p.num_steps * (kTcBK / 8) <= 16 && 2 * p.Npad <= 512) ? 1 : 0;
+  p.nacc = split && !p.merge_corr ? 2 : 1;
   p.acc_stages = 2 * p.nacc * p.Npad <= 512 ? 2 : 1;
-  if (p.acc_stages == 1 && want <= 2 && p.nmain > 1 && 2 * (p.nmain - 1 + corr) * p.Npad <= 512) {
-    p.nmain--;
-    p.nacc--;
-    p.acc_stages = 2;
-  }
   p.tmem_cols = 32;
   while ((int)p.tmem_cols < p.acc_stages * p.nacc * p.Npad) p.tmem_cols <<= 1;
-  static const bool no_stack = getenv("YNB_TC_NO_STACK") != nullptr;
-  p.stack_b = (split && !no_stack && p.nmain == 1 && p.nacc == 2 && 2 * p.Npad <= 256 && (2 * p.Npad) % 16 == 0) ? 1 : 0;
+  p.stack_b = (p.nacc == 2 && 2 * p.Npad <= 256 && (2 * p.Npad) % 16 == 0) ? 1 : 0;
 }
 
 // Picks stages / residency for the smem budget.  Returns false if nothing fits.
@@ -905,8 +862,7 @@ inline bool tc_plan_smem(TcGemmLaunch& L) {
     for (int stages = kTcMaxStages; stages >= 2; --stages) {
       if (stages > p.num_steps * 4 && stages > 2) continue;
       TcSmemLayout lay = tc_smem_layout(p.Npad, p.num_steps, stages, resident != 0, split);
-      static const bool res2 = getenv("YNB_TC_RES2") != nullptr;   // experiment: W resident with 2 A stages
-      if (lay.total <= (uint32_t)kTcSmemBudget && (resident == 0 || stages >= 3 || p.num_steps <= 2 || res2)) {
+      if (lay.total <= (uint32_t)kTcSmemBudget && (resident == 0 || stages >= 3 || p.num_steps <= 2)) {
         p.num_stages = stages;
         p.w_resident = resident;
         L.smem = lay.total;

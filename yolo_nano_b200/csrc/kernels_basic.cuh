@@ -658,40 +658,40 @@ inline cudaError_t launch_dwconv3x3(const float* in, int in_ld, int in_off, floa
 }
 
 // =====================================================================================
-// Pass-through half of a stride-1 ShuffleNetV2 unit: out[m, slot(2i)] = in[m, i], i < half.
-// Together with the branch-2 epilogue (which writes slot(2i+1)) this IS
+// Pass-through half of a stride-1 ShuffleNetV2 unit: out[m, 2i] = in[m, i], i < half.
+// Together with the branch-2 epilogue (which writes channel 2i+1) this IS
 // torch.cat + channel_shuffle (backbone/shufflenetv2.py:70-76, 14-28): no shuffle copy.
 // =====================================================================================
 __global__ void __launch_bounds__(256)
 interleave_copy_kernel(const float* __restrict__ in, int in_ld, float* __restrict__ out, int out_ld,
-                       ChanMap omap, int64_t pixels, int half) {
+                       int64_t pixels, int half) {
   const int64_t total = pixels * half;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (int64_t)gridDim.x * blockDim.x) {
     int c = (int)(i % half);
     int64_t m = i / half;
-    out[m * out_ld + omap.slot(2 * c)] = __ldg(in + m * in_ld + c);
+    out[m * out_ld + 2 * c] = __ldg(in + m * in_ld + c);
   }
 }
 
 inline cudaError_t launch_interleave_copy(const float* in, int in_ld, float* out, int out_ld,
-                                          ChanMap omap, int64_t pixels, int half, cudaStream_t st) {
+                                          int64_t pixels, int half, cudaStream_t st) {
   int64_t blocks = (pixels * half + 255) / 256;
   int64_t cap = (int64_t)kNumSMs * 16;
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
-  interleave_copy_kernel<<<(unsigned)blocks, 256, 0, st>>>(in, in_ld, out, out_ld, omap, pixels, half);
+  interleave_copy_kernel<<<(unsigned)blocks, 256, 0, st>>>(in, in_ld, out, out_ld, pixels, half);
   YNB_COUNT_LAUNCH();
   return cudaGetLastError();
 }
 
 // =====================================================================================
-// Tap / parity hook: internal NHWC (with channel map) -> canonical NCHW.
+// Tap / parity hook: internal NHWC -> canonical NCHW.
 // Tiled transpose through shared memory: coalesced on both sides.
 // =====================================================================================
 template <typename E>
 __global__ void __launch_bounds__(256)
-nhwc_to_nchw_kernel(const E* __restrict__ in, int in_ld, ChanMap imap, float* __restrict__ out,
+nhwc_to_nchw_kernel(const E* __restrict__ in, int in_ld, float* __restrict__ out,
                     int C, int HW) {
   __shared__ float tile[32][33];
   const int b = blockIdx.z;
@@ -700,7 +700,7 @@ nhwc_to_nchw_kernel(const E* __restrict__ in, int in_ld, ChanMap imap, float* __
   for (int r = ty; r < 32; r += 8) {
     int p = p0 + r, c = c0 + tx;
     float v = 0.0f;
-    if (p < HW && c < C) v = to_float(in[((size_t)b * HW + p) * in_ld + imap.slot(c)]);
+    if (p < HW && c < C) v = to_float(in[((size_t)b * HW + p) * in_ld + c]);
     tile[r][tx] = v;
   }
   __syncthreads();
@@ -710,11 +710,11 @@ nhwc_to_nchw_kernel(const E* __restrict__ in, int in_ld, ChanMap imap, float* __
   }
 }
 
-inline cudaError_t launch_nhwc_to_nchw(const void* in, int in_ld, ChanMap imap, float* out,
+inline cudaError_t launch_nhwc_to_nchw(const void* in, int in_ld, float* out,
                                        int batch, int C, int HW, cudaStream_t st, bool in_bf16 = false) {
   dim3 grid((HW + 31) / 32, (C + 31) / 32, batch);
-  if (in_bf16) nhwc_to_nchw_kernel<<<grid, 256, 0, st>>>(static_cast<const bf16*>(in), in_ld, imap, out, C, HW);
-  else nhwc_to_nchw_kernel<<<grid, 256, 0, st>>>(static_cast<const float*>(in), in_ld, imap, out, C, HW);
+  if (in_bf16) nhwc_to_nchw_kernel<<<grid, 256, 0, st>>>(static_cast<const bf16*>(in), in_ld, out, C, HW);
+  else nhwc_to_nchw_kernel<<<grid, 256, 0, st>>>(static_cast<const float*>(in), in_ld, out, C, HW);
   YNB_COUNT_LAUNCH();
   return cudaGetLastError();
 }

@@ -699,13 +699,15 @@ inline int dw_bwd_chunks(int B, int h_out, int w_out) {
 // 128 x 128 tile of (n, k)); 16-pixel slabs of dOut and in go through shared memory (next slab
 // prefetched into registers while the current one is multiplied), each thread owns an 8 x 8 register
 // tile (two 4-wide column groups 64 apart: conflict-free 16-byte shared loads).  partial[chunk][N][K] is
-// summed in fixed order by reduce_partials_kernel.
+// summed in fixed order by reduce_partials_kernel.  This kernel serves the views that are not 16-byte aligned
+// (aligned ones go to the cp.async variant below): scalar loads, through the read-only path (__ldg: 133 registers,
+// plain loads 137, CUDA 12.9).
 constexpr int kPwBwdTile = 128;
 constexpr int kPwBwdSlab = 16;
 __global__ void __launch_bounds__(256) pwconv_bwd_weight_kernel(const float* __restrict__ dout, int do_ld, int do_off,
                                                                 const float* __restrict__ in, int in_ld, int in_off,
                                                                 float* __restrict__ partial_w, float* __restrict__ partial_b,
-                                                                long long M, int K, int N, long long m_per_chunk, int vec) {
+                                                                long long M, int K, int N, long long m_per_chunk) {
   __shared__ __align__(16) float sd[kPwBwdSlab][kPwBwdTile];
   __shared__ __align__(16) float sx[kPwBwdSlab][kPwBwdTile];
   const int n0 = blockIdx.y * kPwBwdTile, k0 = blockIdx.z * kPwBwdTile;
@@ -729,19 +731,14 @@ __global__ void __launch_bounds__(256) pwconv_bwd_weight_kernel(const float* __r
       if (mm < m1) {
         const float* dp = dout + mm * do_ld + do_off + n0 + lc;
         const float* xp = in + mm * in_ld + in_off + k0 + lc;
-        if (vec) {
-          if (n0 + lc < N) d = *reinterpret_cast<const float4*>(dp);
-          if (k0 + lc < K) x = *reinterpret_cast<const float4*>(xp);
-        } else {
-          if (n0 + lc < N) d.x = dp[0];
-          if (n0 + lc + 1 < N) d.y = dp[1];
-          if (n0 + lc + 2 < N) d.z = dp[2];
-          if (n0 + lc + 3 < N) d.w = dp[3];
-          if (k0 + lc < K) x.x = xp[0];
-          if (k0 + lc + 1 < K) x.y = xp[1];
-          if (k0 + lc + 2 < K) x.z = xp[2];
-          if (k0 + lc + 3 < K) x.w = xp[3];
-        }
+        if (n0 + lc < N) d.x = __ldg(dp);
+        if (n0 + lc + 1 < N) d.y = __ldg(dp + 1);
+        if (n0 + lc + 2 < N) d.z = __ldg(dp + 2);
+        if (n0 + lc + 3 < N) d.w = __ldg(dp + 3);
+        if (k0 + lc < K) x.x = __ldg(xp);
+        if (k0 + lc + 1 < K) x.y = __ldg(xp + 1);
+        if (k0 + lc + 2 < K) x.z = __ldg(xp + 2);
+        if (k0 + lc + 3 < K) x.w = __ldg(xp + 3);
       }
       pd[h] = d; px[h] = x;
     }

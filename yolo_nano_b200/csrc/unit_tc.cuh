@@ -2,7 +2,7 @@
 // output never reaches HBM):
 //
 //   stride-1 ShuffleNetV2 unit (backbone/shufflenetv2.py:53-63, 70-76):
-//       mid1 --dw3x3+BN--> (smem) --pw+BN+ReLU--> out[slot(2i+1)],  x1[i] -> out[slot(2i)]
+//       mid1 --dw3x3+BN--> (smem) --pw+BN+ReLU--> out[2i+1],  x1[i] -> out[2i]
 //   detection-head pair (models/yolo_nano.py:50-58):
 //       x --dw3x3+BN+Leaky--> (smem) --pw+BN+Leaky--> out
 //
@@ -51,19 +51,17 @@ struct DwPwParams {
   int N, Npad;
   int mode;           // YNB_GEMM_TC_3XTF32 | YNB_GEMM_TC_TF32
   int w_resident, a_stages, raw_stages;
-  int prefetch_tiles; // L2 prefetch distance of the raw tiles, in tiles of this CTA (0: off)
   int pass_blocks;    // 32-channel blocks of the pass-through half to prefetch into L2 per tile (0: none)
-  int tma_out;        // gap-free output layout: every warp's staging box leaves through ONE TMA tensor store (tmOut)
+  int tma_out;        // every warp's staging box leaves through ONE TMA tensor store (tmOut)
   uint32_t tmem_cols;
   const float* dw_w;  // [9][C4] tap-major, BN folded
   const float* dw_b;  // [C4]
   int dw_act;
   float* out;
   int out_ld, out_off;
-  ChanMap omap;
   const float* bias;
   int act;
-  const float* pass;  // stride-1 unit: x1 (same pixels, N channels) -> out[slot(2i)]; conv -> out[slot(2i+1)]
+  const float* pass;  // stride-1 unit: x1 (same pixels, N channels) -> out[2i]; conv -> out[2i+1]
   int pass_ld;
   int* err_flag;
   long long* trace;   // debug timeline (tools/gpu_dp_trace.py): CTA 0 stores clock64 at [role][local tile][chunk]
@@ -206,19 +204,6 @@ dwpw_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__
         // the pass-through half of this tile is read by the epilogue a few microseconds from now: pull it into L2
 #pragma unroll 1
         for (int cb = 0; cb < p.pass_blocks; ++cb) ptx::tma_prefetch_4d(&tmPass, cb * CH, x0, y0, b);
-        // A TMA box takes ~4 k cycles from issue to landing when it comes from HBM (measured, tools/gpu_dp_trace.py)
-        // and only raw_stages x 26 KB fit in flight: the HBM rate would be latency-bound.  Pull the tile this CTA
-        // loads `pf` tiles from now into L2 (no shared memory needed), so that its loads are L2 hits.
-        if (p.prefetch_tiles > 0) {
-          const int64_t tp = tile + (int64_t)p.prefetch_tiles * gridDim.x;
-          if (tp < p.num_tiles) {
-            const int bp = (int)(tp / per_img);
-            const int rp = (int)(tp - (int64_t)bp * per_img);
-            const int yp = (rp / p.tiles_x) * TH, xp = (rp % p.tiles_x) * TW;
-#pragma unroll 1
-            for (int kc = 0; kc < p.num_chunks; ++kc) ptx::tma_prefetch_4d(&tmIn, kc * CH, xp - 1, yp - 1, bp);
-          }
-        }
         for (int kc = 0; kc < p.num_chunks; ++kc) {
           ok = ptx::mbar_wait(&raw_empty[r], ph ^ 1, p.err_flag, 1);
           if (!ok) break;
@@ -412,14 +397,13 @@ dwpw_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__
     // The thread that owns a tile row builds 128 bytes of its OUTPUT row in the warp's swizzled staging box
     // (interleaved with the pass-through half for ShuffleNet units) — no transposition: it owns the same row
     // of the accumulator — and the warp then copies the box out with 16-byte accesses (whole 128-byte row
-    // segments per instruction); across a layout gap the unit is one (x1, conv) pair.
+    // segments per instruction).
     const int group = warp >> 2, q = warp & 3;            // group g drains the tiles with (local index & 1) == g
     const int row = q * 32 + lane;
     const float slope = p.act == YNB_ACT_RELU ? 0.0f : (p.act == YNB_ACT_LEAKY ? 0.1f : 1.0f);
     uint8_t* sbox = smem + lay.stg_off + warp * 4096;
     const int sw = lane & 7;
     const int yy = row >> p.lgTW, xx = row & (TW - 1);
-    const bool gap = p.omap.gap != 0;
     constexpr int BOX = 128 / (int)sizeof(E);              // output elements per row and box: 32 | 64
     constexpr int CPB = kPass ? BOX / 2 : BOX;             // accumulator columns per box: 16/32 | 32/64
     constexpr int EPC = 16 / (int)sizeof(E);               // elements per 16-byte chunk: 4 | 8
@@ -572,38 +556,16 @@ dwpw_tc_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__
           }
           continue;
         }
-        if (!gap) {
-          const int ch = lane & 7;
-          const int jc = j0 + EPC * ch;
-#pragma unroll
-          for (int k = 0; k < 8; ++k) {
-            const int r = (lane >> 3) + 4 * k;
-            const int oo = __shfl_sync(0xffffffffu, ooff, r);
-            const uint4 val = *reinterpret_cast<const uint4*>(sbox + r * 128 + ((ch ^ (r & 7)) << 4));
-            if (oo >= 0 && jc < out_cols) *reinterpret_cast<uint4*>(outp + oo + p.out_off + jc) = val;
-          }
-        } else if (!kBf16) {
-          const int pr = lane & 15;        // 8-byte (x1, conv) pair
-          const int jc = j0 + 2 * pr;
-          const int col = p.omap.slot(p.out_off + jc);
-#pragma unroll
-          for (int k = 0; k < 16; ++k) {
-            const int r = (lane >> 4) + 2 * k;
-            const int oo = __shfl_sync(0xffffffffu, ooff, r);
-            const uint2 val =
-                *reinterpret_cast<const uint2*>(sbox + r * 128 + ((((pr >> 1) ^ (r & 7)) << 4) | ((pr & 1) << 3)));
-            if (oo >= 0 && jc < out_cols) *reinterpret_cast<uint2*>(outp + oo + col) = val;
-          }
-        } else {
-          const int jc = j0 + 2 * lane;    // bf16: 4-byte (x1, conv) pair per lane, one 128-byte row per instruction
-          const int col = p.omap.slot(p.out_off + jc);
+        // Per-lane copy-out, for outputs the tensor map cannot describe: lanes 0-15 store two 128-byte row segments per
+        // instruction.  (Full-warp stores of four rows cost the bf16 instantiations two more registers, CUDA 12.9.)
+        const int ch = lane & 7;
+        const int jc = j0 + EPC * ch;
 #pragma unroll 8
-          for (int r = 0; r < 32; ++r) {
-            const int oo = __shfl_sync(0xffffffffu, ooff, r);
-            const uint32_t val =
-                *reinterpret_cast<const uint32_t*>(sbox + r * 128 + ((((lane >> 2) ^ (r & 7)) << 4) | ((lane & 3) << 2)));
-            if (oo >= 0 && jc < out_cols) *reinterpret_cast<uint32_t*>(outp + oo + col) = val;
-          }
+        for (int k = 0; k < 16; ++k) {
+          const int r = ((lane >> 3) & 1) + 2 * k;
+          const int oo = __shfl_sync(0xffffffffu, ooff, r);
+          const uint4 val = *reinterpret_cast<const uint4*>(sbox + r * 128 + ((ch ^ (r & 7)) << 4));
+          if (lane < 16 && oo >= 0 && jc < out_cols) *reinterpret_cast<uint4*>(outp + oo + p.out_off + jc) = val;
         }
         __syncwarp();
       }
@@ -648,8 +610,6 @@ inline bool plan_dwpw(DwPwLaunch& L, const void* in, int in_ld, int B, int H, in
   {   // 16 x 8 or 32 x 4 output pixels per tile: whichever covers the map with fewer tiles
     const int t16 = ((W + 15) / 16) * ((H + 7) / 8), t32 = ((W + 31) / 32) * ((H + 3) / 4);
     p.lgTW = t32 < t16 ? 5 : 4;
-    static const int force = getenv("YNB_DP_LGTW") ? atoi(getenv("YNB_DP_LGTW")) : 0;      // experiment knob
-    if (force == 4 || force == 5) p.lgTW = force;
   }
   const int TW = 1 << p.lgTW, TH = kTcBM >> p.lgTW;
   p.tiles_x = (W + TW - 1) / TW;
@@ -665,10 +625,8 @@ inline bool plan_dwpw(DwPwLaunch& L, const void* in, int in_ld, int B, int H, in
   // Shared memory: a 2-deep A ring is enough (it only decouples the depthwise producers from the MMAs, both
   // on chip); everything else goes to the raw ring — the TMA bytes in flight per SM are what bounds the HBM rate.
   bool found = false;
-  static const int wres = getenv("YNB_DP_WRES") ? atoi(getenv("YNB_DP_WRES")) : -1;          // experiment knob: 0 | 1
   for (int raw = kDpMaxRawStages; raw >= 2 && !found; --raw)
     for (int resident = 1; resident >= 0 && !found; --resident) {
-      if (wres >= 0 && resident != wres) continue;
       DpSmemLayout lay = dp_smem_layout(p.Npad, p.num_chunks, p.lgTW, 2, raw, resident != 0, split, chunk_ch);
       if (lay.total <= (uint32_t)kTcSmemBudget) {
         p.a_stages = 2; p.raw_stages = raw; p.w_resident = resident; L.smem = lay.total;
@@ -676,10 +634,6 @@ inline bool plan_dwpw(DwPwLaunch& L, const void* in, int in_ld, int B, int H, in
       }
     }
   if (!found) return false;
-  {
-    static const int pf = getenv("YNB_DP_PREFETCH") ? atoi(getenv("YNB_DP_PREFETCH")) : 0;   // measured: no gain (DESIGN 4.5)
-    p.prefetch_tiles = pf;
-  }
   const int epc = 16 / es;                // elements per 16 bytes
   if ((reinterpret_cast<uintptr_t>(p.out) & 15u) || (p.out_ld % epc) || (p.out_off % epc)) return false;
   p.pass_blocks = 0;
@@ -691,13 +645,9 @@ inline bool plan_dwpw(DwPwLaunch& L, const void* in, int in_ld, int B, int H, in
   // the raw tile is NOT swizzled: the depthwise threads that read one tile row together cover its 128 bytes
   // (lane = channel group fastest), so plain rows are conflict-free and need no XOR per load
   if (!make_tmap_nhwc(&L.tmIn, in, C4, W, H, B, in_ld, TW + 2, TH + 2, is_bf16, false)) return false;
-  p.tma_out = 0;
   {
-    static const bool no_ts = getenv("YNB_DP_NO_TMA_STORE") != nullptr;                     // experiment knob
     const int out_cols = p.pass ? 2 * p.N : (p.N + epc - 1) / epc * epc;
-    if (!no_ts && p.omap.gap == 0 && p.out_off == 0 &&
-        make_tmap_nhwc(&L.tmOut, p.out, out_cols, W, H, B, p.out_ld, TW, 32 / TW, is_bf16))
-      p.tma_out = 1;
+    p.tma_out = p.out_off == 0 && make_tmap_nhwc(&L.tmOut, p.out, out_cols, W, H, B, p.out_ld, TW, 32 / TW, is_bf16);
   }
   L.w = w;
   L.grid = (unsigned)std::min<int64_t>(p.num_tiles, kNumSMs);

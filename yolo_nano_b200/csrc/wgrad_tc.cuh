@@ -351,9 +351,8 @@ inline cudaError_t launch_pw_wgrad_tc(WgradParams p, int chunks, cudaStream_t st
   const long long total_steps = (p.M + kWgStepPix - 1) / kWgStepPix;
   p.steps_per_chunk = (total_steps + chunks - 1) / chunks;
   const size_t stage = 2 * kWgABytes + 2 * (size_t)kpad * 128;
-  static const bool no_raw = getenv("YNB_WGRAD_NO_RAW") != nullptr;
-  if (kpad == 128 && !no_raw) { p.stages = 2; p.raw_slots = 3; }       // 2 x 64 KB operand stages + 3 x 32 KB raw slots
-  else { p.stages = kpad == 128 ? 3 : 2; p.raw_slots = 0; }
+  p.stages = 2;                                   // 2 operand stages (64 KB each at kpad 128)
+  p.raw_slots = kpad == 128 ? 3 : 0;              // + 3 x 32 KB raw slots at kpad 128
   const size_t smem = stage * p.stages + (size_t)p.raw_slots * 32768 + 1024;
   dim3 grid(chunks, (p.N + 127) / 128);
   cudaError_t e;

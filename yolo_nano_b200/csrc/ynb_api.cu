@@ -43,7 +43,6 @@ struct Tensor {
   int C = 0;        // logical channels
   int ld = 0;       // elements per pixel
   int H = 0, W = 0;
-  ChanMap map = {INT_MAX, 0};
   size_t floats_per_image() const { return (size_t)H * W * ld; }
   void* at(int off = 0) const { return reinterpret_cast<char*>(p) + (size_t)off * es; }   // address of element `off`
 };
@@ -51,7 +50,7 @@ struct Tensor {
 // How a conv's input channels are laid out physically (static per conv).
 struct InLayout {
   int ktot;       // physical width read by the conv (multiple of 4)
-  ChanMap map;    // logical k -> physical slot inside the view
+  int shift;      // logical input channel k sits at position k + shift of the view
 };
 
 struct PackedConv {
@@ -204,54 +203,38 @@ struct CounterScope {
 };
 
 // ---- static layout knowledge -----------------------------------------------------------
-// TMA views and 16-byte loads must start 16-byte aligned: 4 floats or 8 bf16.  Earlier layout (YNB_GAP_STAGE2=1 keeps
-// it): a gap between the halves — float stage 2 = [58 | 2 pad | 58 | 2 pad] (ld 120), bf16 stage 2 = [58 | 6 | 58 | 6]
-// (ld 128), bf16 stage 3 = [116 | 4 | 116 | 4] (ld 240); everything else dense.
-struct StageLayout { int ld; ChanMap map; };
-// Stage outputs are DENSE (float stage 2: 116 channels; bf16 stage 2: 116 + 4 zero pad, stage 3: 232).  Where the second
-// half does not start on a 16-byte boundary (h = 58 floats, 58 / 116 bf16), the one conv that reads only x2 (branch2[0]
-// of the stride-1 units) reads the aligned window that starts h % a channels earlier, with its weights shifted by as
-// many input positions (zero weight on the leading channels): see x2_window() / in_layout().  A dense layout lets the
-// fused unit tails leave through TMA tensor stores (a gap between the halves cannot be stored that way).
-static bool dense_stage2() {
-  static const bool off = getenv("YNB_GAP_STAGE2") != nullptr;      // experiment knob: the round-2a gap layout
-  return !off;
-}
-StageLayout stage_layout(bool bf, int si) {
-  const int cout = stage_channels()[si + 1], h = cout / 2, a = bf ? 8 : 4;
-  const int hp = round_up(h, a);
-  if (hp == h) return {cout, dense_map()};
-  if (dense_stage2()) return {round_up(cout, a), dense_map()};     // channels >= cout: zero pad at the END of the row
-  return {2 * hp, ChanMap{h, hp - h}};
-}
-// Aligned window over the second half of a dense stage output with h % a != 0: start channel and weight shift.
+// TMA views and 16-byte loads must start 16-byte aligned: 4 floats or 8 bf16.  Stage outputs are DENSE (float stage 2:
+// 116 channels; bf16 stage 2: 116 + 4 zero pad, stage 3: 232), any pad at the END of the row.  Where the second half
+// does not start on a 16-byte boundary (h = 58 floats, 58 / 116 bf16), the one conv that reads only x2 (branch2[0] of
+// the stride-1 units) reads the aligned window that starts h % a channels earlier, with its weights shifted by as many
+// input positions (zero weight on the leading channels): see x2_window() / in_layout().  A dense layout lets the fused
+// unit tails leave through TMA tensor stores.
+int stage_ld(bool bf, int si) { return round_up(stage_channels()[si + 1], bf ? 8 : 4); }
+// Aligned window over the second half of a stage output: start channel and weight shift.
 struct X2Window { int off, shift; };
-X2Window x2_window(const StageLayout& sl, int h, int a) {
-  if (sl.map.gap != 0) return {sl.map.slot(h), 0};
-  return {h - h % a, h % a};
-}
+X2Window x2_window(int h, int a) { return {h - h % a, h % a}; }
 
 // Input layout of conv `name` (see plan_network for the producers).
 InLayout in_layout(const ConvSpec& c, bool bf) {
   const std::string& n = c.name;
-  if (c.kind == kDense3x3) return {c.cin == 3 ? 27 : 9 * c.cin, dense_map()};
+  if (c.kind == kDense3x3) return {c.cin == 3 ? 27 : 9 * c.cin, 0};
   bool reads_c3 = n == "backbone.stage3.0.branch1.0" || n == "backbone.stage3.0.branch1.2" ||
                   n == "backbone.stage3.0.branch2.0" || n == "conv1x1_0.convs.0";
   bool reads_c4 = n == "backbone.stage4.0.branch1.0" || n == "backbone.stage4.0.branch1.2" ||
                   n == "backbone.stage4.0.branch2.0" || n == "conv1x1_1.convs.0";
-  if (reads_c3) { StageLayout L = stage_layout(bf, 0); return {L.ld, L.map}; }
-  if (reads_c4) { StageLayout L = stage_layout(bf, 1); return {L.ld, L.map}; }
-  // branch2[0] of a stride-1 unit reads x2 of its stage's layout: through an aligned, shifted window when that is dense
+  if (reads_c3) return {stage_ld(bf, 0), 0};
+  if (reads_c4) return {stage_ld(bf, 1), 0};
+  // branch2[0] of a stride-1 unit reads x2 of its stage's output: through an aligned, shifted window
   for (int si = 0; si < 3; ++si) {
     const std::string pre = "backbone.stage" + std::to_string(si + 2) + ".";
     if (n.compare(0, pre.size(), pre) == 0 && n.size() > pre.size() + 2 && n[pre.size()] != '0' &&
         n.compare(n.size() - 10, 10, ".branch2.0") == 0) {
       const int a = bf ? 8 : 4;
-      const X2Window w = x2_window(stage_layout(bf, si), c.cin, a);
-      if (w.shift) return {round_up(c.cin + w.shift, a), ChanMap{0, w.shift}};
+      const X2Window w = x2_window(c.cin, a);
+      if (w.shift) return {round_up(c.cin + w.shift, a), w.shift};
     }
   }
-  return {round_up(c.cin, bf ? 8 : 4), dense_map()};
+  return {round_up(c.cin, bf ? 8 : 4), 0};
 }
 
 // ---- weight packing ----------------------------------------------------------------------
@@ -300,7 +283,7 @@ int pack_tc_matrix(ynb_engine* e, TcWeights& t, const float* w, int n, int ktot,
 // The two output branches of a stride-2 ShuffleNetV2 unit as ONE pointwise conv (backbone/shufflenetv2.py:43-49,
 // 57-63, 73-76): A = [branch1 dw output | branch2 dw output] concatenated along K (each padded to whole K chunks),
 // weights block-diagonal with the rows interleaved the way channel_shuffle interleaves the branches:
-//   row slot(2i)   = [ W_branch1.2[i] | 0 ],   row slot(2i+1) = [ 0 | W_branch2.5[i] ]      (+ zero rows on pad slots)
+//   row 2i = [ W_branch1.2[i] | 0 ],   row 2i+1 = [ 0 | W_branch2.5[i] ]      (+ zero rows on the pad at the end)
 // so that torch.cat + channel_shuffle is the GEMM's plain dense output (TMA-store epilogue) instead of two launches
 // with 4-byte scattered stores.  Wider than one MMA tile (stage 4: 464 columns) -> split along N.
 int pack_cat(ynb_engine* e, int si) {
@@ -312,20 +295,20 @@ int pack_cat(ynb_engine* e, int si) {
   const PackedConv& p1 = e->convs[i1];
   const PackedConv& p2 = e->convs[i2];
   const InLayout il1 = in_layout(c1, bf), il2 = in_layout(c2, bf);
-  const StageLayout sl = stage_layout(bf, si);
+  const int ld = stage_ld(bf, si);
   const int ch = bf ? 64 : kTcBK;
   const int k1p = round_up(il1.ktot, ch), k2p = round_up(il2.ktot, ch), ktot = k1p + k2p;
   const int h = c1.cout;
-  std::vector<float> w((size_t)sl.ld * ktot, 0.f), b((size_t)sl.ld, 0.f);
+  std::vector<float> w((size_t)ld * ktot, 0.f), b((size_t)ld, 0.f);
   for (int i = 0; i < h; ++i) {
-    const int r1 = sl.map.slot(2 * i), r2 = sl.map.slot(2 * i + 1);
-    for (int k = 0; k < c1.cin; ++k) w[(size_t)r1 * ktot + il1.map.slot(k)] = p1.w_host[(size_t)i * c1.cin + k];
-    for (int k = 0; k < c2.cin; ++k) w[(size_t)r2 * ktot + k1p + il2.map.slot(k)] = p2.w_host[(size_t)i * c2.cin + k];
+    const int r1 = 2 * i, r2 = 2 * i + 1;
+    for (int k = 0; k < c1.cin; ++k) w[(size_t)r1 * ktot + k + il1.shift] = p1.w_host[(size_t)i * c1.cin + k];
+    for (int k = 0; k < c2.cin; ++k) w[(size_t)r2 * ktot + k1p + k + il2.shift] = p2.w_host[(size_t)i * c2.cin + k];
     b[r1] = p1.b_host[i];
     b[r2] = p2.b_host[i];
   }
-  const int parts = (sl.ld + 239) / 240;                    // N <= 240 per launch (TMEM: 2 x 240 columns in parity mode)
-  const int npart = round_up((sl.ld + parts - 1) / parts, bf ? 8 : 4);
+  const int parts = (ld + 239) / 240;                       // N <= 240 per launch (TMEM: 2 x 240 columns in parity mode)
+  const int npart = round_up((ld + parts - 1) / parts, bf ? 8 : 4);
   for (auto& cc : e->cat[si]) {
     if (cc.pc.b_dev) cudaFree(cc.pc.b_dev);
     if (cc.pc.tc.hi) cudaFree(cc.pc.tc.hi);
@@ -337,7 +320,7 @@ int pack_cat(ynb_engine* e, int si) {
   for (int pi = 0; pi < parts; ++pi) {
     ynb_engine::CatConv& cc = e->cat[si][pi];
     cc.n0 = pi * npart;
-    const int n = std::min(npart, sl.ld - cc.n0);
+    const int n = std::min(npart, ld - cc.n0);
     cc.k1p = k1p; cc.k2p = k2p;
     cc.pc.n = n; cc.pc.ktot = ktot; cc.pc.loaded = true;
     CUDA_TRY(e, cudaMalloc(&cc.pc.b_dev, round_up(n, 4) * 4));
@@ -365,20 +348,20 @@ int pack_conv(ynb_engine* e, int i) {
     pc.n = 24; pc.ktot = 27;
     memcpy(e->stem_w.w, w.data(), sizeof(e->stem_w.w));
     memcpy(e->stem_w.b, b.data(), sizeof(e->stem_w.b));
-  } else if (c.kind == kDw3x3) {                       // [9][C4] by physical slot
+  } else if (c.kind == kDw3x3) {                       // [9][C4] by physical position
     int c4 = il.ktot;
     w.assign(9 * c4, 0.f);
     b.assign(c4, 0.f);
     for (int ch = 0; ch < c.cin; ++ch) {
-      int s = il.map.slot(ch);
+      int s = ch + il.shift;
       for (int t = 0; t < 9; ++t) w[t * c4 + s] = pc.w_host[ch * 9 + t];
       b[s] = pc.b_host[ch];
     }
     pc.n = c4; pc.ktot = 9;
-  } else if (c.kind == kPw1x1) {                       // [N][Ktot] by physical slot
+  } else if (c.kind == kPw1x1) {                       // [N][Ktot] by physical position
     w.assign((size_t)c.cout * il.ktot, 0.f);
     for (int n = 0; n < c.cout; ++n)
-      for (int k = 0; k < c.cin; ++k) w[(size_t)n * il.ktot + il.map.slot(k)] = pc.w_host[(size_t)n * c.cin + k];
+      for (int k = 0; k < c.cin; ++k) w[(size_t)n * il.ktot + k + il.shift] = pc.w_host[(size_t)n * c.cin + k];
     b = pc.b_host;
     pc.n = c.cout; pc.ktot = il.ktot;
   } else {                                             // dense 3x3: [N][tap][cin]
@@ -423,10 +406,10 @@ size_t layout_workspace(ynb_engine* e, int batch, int S, char* base) {
   Bump bump;
   const bool bf = is_bf16(e);
   const int es_act = bf ? 2 : 4, al = bf ? 8 : 4;
-  auto tensor = [&](const std::string& name, int C, int ld, int H, ChanMap map = dense_map(), int es = 0) {
+  auto tensor = [&](const std::string& name, int C, int ld, int H, int es = 0) {
     Tensor t;
     t.es = es ? es : es_act;
-    t.C = C; t.ld = ld; t.H = H; t.W = H; t.map = map;
+    t.C = C; t.ld = ld; t.H = H; t.W = H;
     size_t o = bump.take((size_t)batch * H * H * ld * t.es);
     t.p = base ? reinterpret_cast<float*>(base + o) : nullptr;
     e->taps[name] = t;
@@ -437,21 +420,19 @@ size_t layout_workspace(ynb_engine* e, int batch, int S, char* base) {
   tensor("pool", 24, 24, H1);
   int hin = H1;
   int ld_in = 24;
-  ChanMap map_in = dense_map();
   for (int si = 0; si < 3; ++si) {
     int cout = stage_channels()[si + 1], h = cout / 2, cin = stage_channels()[si];
     int hout = hin / 2;
     std::string st = "stage" + std::to_string(si + 2);
-    const StageLayout sl = stage_layout(bf, si);
+    const int ld = stage_ld(bf, si);
     int ld_h = round_up(h, al);
-    tensor(st + ".b1dw", cin, ld_in, hout, map_in);                            // branch1 dw output (layout of its input)
+    tensor(st + ".b1dw", cin, ld_in, hout);                                    // branch1 dw output (layout of its input)
     tensor(st + ".b2pw", h, ld_h, hin);                                        // branch2 first pw @ input res
     tensor(st + ".mid1", h, ld_h, hout);                                       // pw1 / dw scratch
     tensor(st + ".mid2", h, ld_h, hout);
-    for (int bi = 0; bi < stage_repeats()[si]; ++bi) tensor(st + "." + std::to_string(bi), cout, sl.ld, hout, sl.map);
+    for (int bi = 0; bi < stage_repeats()[si]; ++bi) tensor(st + "." + std::to_string(bi), cout, ld, hout);
     hin = hout;
-    ld_in = sl.ld;
-    map_in = sl.map;
+    ld_in = ld;
   }
   const int H3 = S / 8, H4 = S / 16, H5 = S / 32;
   const int hs[3] = {H3, H4, H5};
@@ -466,7 +447,7 @@ size_t layout_workspace(ynb_engine* e, int batch, int S, char* base) {
     tensor("head" + std::to_string(l) + ".a", 96, 96, hs[l]);
     tensor("head" + std::to_string(l) + ".b", 96, 96, hs[l]);
     tensor("head" + std::to_string(l) + ".c", 96, 96, hs[l]);
-    e->raw[l] = tensor(pn[l], ch, round_up(ch, 4), hs[l], dense_map(), 4);    // raw head maps stay float32
+    e->raw[l] = tensor(pn[l], ch, round_up(ch, 4), hs[l], 4);    // raw head maps stay float32
   }
   // aliases used as taps
   e->taps["c3"] = e->taps["stage2.3"];
@@ -511,7 +492,7 @@ int ensure_workspace(ynb_engine* e, int batch) {
   if (e->ws) { cudaFree(e->ws); e->ws = nullptr; }
   size_t bytes = layout_workspace(e, nb, e->S, nullptr);
   CUDA_TRY(e, cudaMalloc(&e->ws, bytes));
-  // zero once: channel pads (58->60, gap slots) are never written afterwards and must be 0
+  // zero once: channel pads (58->60, the pad at the end of a bf16 stage-2 row) are never written afterwards and must be 0
   CUDA_TRY(e, cudaMemset(e->ws, 0, bytes));
   layout_workspace(e, nb, e->S, e->ws);
   e->ws_bytes = bytes;
@@ -544,10 +525,9 @@ struct Planner {
     const bool bf = is_bf16(e);
     const double bytes = (double)in.es * c.cin * (px_in + px_out) + 40.0 * c.cin, flops = 18.0 * c.cin * px_out;
     // product path: halo tiles through TMA; register-tiled global loads if the view is not 16-byte aligned
-    static const bool no_tma = getenv("YNB_DW_NO_TMA") != nullptr;
     e->dw_maps.emplace_back();
     CUtensorMap* tm = &e->dw_maps.back();
-    if ((!no_tma || bf) && make_tmap_dw(tm, in.p, in.ld, in_off, B, in.H, in.W, c4, stride, bf)) {
+    if (make_tmap_dw(tm, in.p, in.ld, in_off, B, in.H, in.W, c4, stride, bf)) {
       plan->net.push_back({name, "dwconv3x3", bytes, flops, [=](cudaStream_t st) {
         return launch_dwconv3x3_tma(*tm, out.p, out.ld, 0, w, b, B_, in.H, in.W, c4, stride, act, st, false, bf);
       }});
@@ -559,20 +539,20 @@ struct Planner {
     }});
   }
 
-  // Pass-through half of a stride-1 unit: out[slot(2i)] = x[i].  HBM-bound copy that only
+  // Pass-through half of a stride-1 unit: out[2i] = x[i].  HBM-bound copy that only
   // depends on the previous unit, so it runs on the side stream next to the unit's convs.
   void passthrough(const std::string& name, const Tensor& x, const Tensor& out, int half) {
     int64_t M = (int64_t)B * x.H * x.W;
     Tensor ps = x, o = out;
     Op op{name + "+passthrough", "interleave_copy", 8.0 * M * half, 0.0, [=](cudaStream_t st) {
-      return launch_interleave_copy(ps.p, ps.ld, o.p, o.ld, o.map, M, half, st);
+      return launch_interleave_copy(ps.p, ps.ld, o.p, o.ld, M, half, st);
     }};
     op.side = true;
     plan->net.push_back(op);
   }
 
-  // pointwise conv: in view (off, ktot) -> out (off, step, map)
-  // `pass`: stride-1 unit tail — out[slot(2i)] = pass[i], out[slot(2i+1)] = conv[i]
+  // pointwise conv: in view (off, ktot) -> out (off, step)
+  // `pass`: stride-1 unit tail — out[2i] = pass[i], out[2i+1] = conv[i]
   void pw(const std::string& name, const Tensor& in, int in_off, const Tensor& out, int out_off, int out_step,
           bool join = false, const Tensor* pass = nullptr, const TcGemmParams::Decode* dec = nullptr) {
     const PackedConv& pc = conv(name);
@@ -587,7 +567,7 @@ struct Planner {
       GemmParams g{};
       g.a = in.p; g.a_ld = in.ld; g.a_off = in_off; g.a2 = nullptr; g.a2_mode = 0;
       g.w = pc.w_dev; g.bias = pc.b_dev; g.out = out.p; g.out_ld = out.ld;
-      g.out_off = out_off; g.out_step = out_step; g.omap = out.map;
+      g.out_off = out_off; g.out_step = out_step;
       g.M = M; g.N = pc.n; g.Ktot = pc.ktot; g.act = c.act;
       if (pass) { g.out_off = 1; g.out_step = 2; }
       Op op{name, "pw_ffma", abytes, aflops, [=](cudaStream_t st) { return launch_gemm_ffma(g, false, st); }};
@@ -615,7 +595,7 @@ struct Planner {
     // raw-map parity tests measure exactly the sums the fused decode epilogue consumes
     tc_plan_tmem(p, name.size() > 2 && name.compare(0, 8, "head_det") == 0 && name.compare(name.size() - 2, 2, ".4") == 0);
     p.a_box_bytes = kTcAStageBytes;
-    p.out = out.p; p.out_ld = out.ld; p.out_off = out_off; p.out_step = out_step; p.omap = out.map;
+    p.out = out.p; p.out_ld = out.ld; p.out_off = out_off; p.out_step = out_step;
     p.bias = pc.b_dev; p.act = c.act;
     p.pass = pass ? pass->p : nullptr; p.pass_ld = pass ? pass->ld : 0;
     p.err_flag = e->d_err;
@@ -624,7 +604,7 @@ struct Planner {
       L.dec_classes = e->cfg.num_classes;
     }
     const int oal = 16 / out.es;                                // output elements per 16 bytes
-    p.tma_store = (!dec && !pass && out_step == 1 && out.map.gap == 0 && out_off % oal == 0 && out.ld % oal == 0) ? 1 : 0;
+    p.tma_store = (!dec && !pass && out_step == 1 && out_off % oal == 0 && out.ld % oal == 0) ? 1 : 0;
     if (p.tma_store && !make_tmap_out(&L.tmOut, out.at(out_off), (uint64_t)round_up(pc.n, oal), (uint64_t)M,
                                       (uint64_t)out.ld, out.es == 2)) {
       error = "cuTensorMapEncodeTiled failed for output of " + name;
@@ -646,10 +626,9 @@ struct Planner {
   }
 
   // The two output convs of a stride-2 unit as one GEMM over K = [b1dw | mid2] (pack_cat): plain dense output.
-  // Returns false when the unit keeps its two strided-store GEMMs (FFMA cross-check mode, switched off).
+  // Returns false when the unit keeps its two strided-store GEMMs (FFMA cross-check mode).
   bool catpw(int si, const std::string& unit, const Tensor& b1dw, const Tensor& mid2, const Tensor& out) {
-    static const bool off = getenv("YNB_NO_CAT_GEMM") != nullptr;
-    if (off || e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA || e->cat[si].empty()) return false;
+    if (e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA || e->cat[si].empty()) return false;
     const bool bf = is_bf16(e);
     const int64_t M = (int64_t)B * out.H * out.W;
     const ConvSpec& c1 = spec(unit + "branch1.2");
@@ -674,7 +653,7 @@ struct Planner {
       p.N = cc.pc.n; p.Npad = cc.pc.tc.Npad;
       tc_plan_tmem(p);
       p.a_box_bytes = kTcAStageBytes;
-      p.out = out.p; p.out_ld = out.ld; p.out_off = cc.n0; p.out_step = 1; p.omap = dense_map();
+      p.out = out.p; p.out_ld = out.ld; p.out_off = cc.n0; p.out_step = 1;
       p.bias = cc.pc.b_dev; p.act = c1.act;
       p.err_flag = e->d_err;
       p.tma_store = 1;
@@ -699,11 +678,10 @@ struct Planner {
   }
 
   // Fused depthwise 3x3 (stride 1) -> pointwise conv in ONE launch (unit_tc.cuh); `pass` as in pw().
-  // Returns false when the pair has to stay unfused (FFMA cross-check mode, shape does not fit, switched off).
+  // Returns false when the pair has to stay unfused (FFMA cross-check mode, shape does not fit).
   bool dwpw(const std::string& dw_name, const std::string& pw_name, const Tensor& in, const Tensor& out,
             const Tensor* pass) {
-    static const bool off = getenv("YNB_NO_FUSED_DWPW") != nullptr;
-    if (off || e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA) return false;
+    if (e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA) return false;
     const PackedConv& dc = conv(dw_name);
     const PackedConv& pc = conv(pw_name);
     const ConvSpec& ds = spec(dw_name);
@@ -714,7 +692,7 @@ struct Planner {
     DwPwParams& p = L.p;
     memset(&p, 0, sizeof(p));
     p.dw_w = dc.w_dev; p.dw_b = dc.b_dev; p.dw_act = ds.act;
-    p.out = out.p; p.out_ld = out.ld; p.out_off = 0; p.omap = out.map;
+    p.out = out.p; p.out_ld = out.ld; p.out_off = 0;
     p.bias = pc.b_dev; p.act = ps.act;
     p.pass = pass ? pass->p : nullptr; p.pass_ld = pass ? pass->ld : 0;
     p.err_flag = e->d_err;
@@ -750,17 +728,16 @@ struct Planner {
       g.a2 = a2 ? a2->p : nullptr; g.a2_ld = a2 ? a2->ld : 0; g.a2_mode = a2 ? a2_mode : 0;
       g.H = a.H; g.W = a.W; g.C = c.cin;
       g.w = pc.w_dev; g.bias = pc.b_dev; g.out = out.p; g.out_ld = out.ld; g.out_off = 0; g.out_step = 1;
-      g.omap = dense_map(); g.M = M; g.N = pc.n; g.Ktot = pc.ktot; g.act = c.act;
+      g.M = M; g.N = pc.n; g.Ktot = pc.ktot; g.act = c.act;
       plan->net.push_back({name, "conv3x3_ffma", 4.0 * M * (c.cin + c.cout) + a2bytes + wbytes, aflops,
                            [=](cudaStream_t st) { return launch_gemm_ffma(g, true, st); }});
       return;
     }
     // tensor-core path: materialise the sum once (HBM-bound elementwise), then 9 shifted TMA boxes
     Tensor src = a;
-    static const bool no_presplit = getenv("YNB_TC_NO_PRESPLIT") != nullptr;
     // fp32-parity mode: the merge kernel writes the sum as exact-tf32 hi + lo planes once, instead of the
     // GEMM splitting every element nine times (once per tap)
-    const bool presplit = a2 != nullptr && e->cfg.gemm_mode == YNB_GEMM_TC_3XTF32 && !no_presplit;
+    const bool presplit = a2 != nullptr && e->cfg.gemm_mode == YNB_GEMM_TC_3XTF32;
     if (a2) {
       Tensor a_ = a, a2_ = *a2, s_ = sum, sl_ = sum_lo;
       int B_ = B;
@@ -790,7 +767,7 @@ struct Planner {
     p.N = pc.n; p.Npad = pc.tc.Npad;
     tc_plan_tmem(p);
     p.a_box_bytes = (uint32_t)(p.TH * p.TW * 128);
-    p.out = out.p; p.out_ld = out.ld; p.out_off = 0; p.out_step = 1; p.omap = dense_map();
+    p.out = out.p; p.out_ld = out.ld; p.out_off = 0; p.out_step = 1;
     p.bias = pc.b_dev; p.act = c.act;
     p.err_flag = e->d_err;
     if (!make_tmap_nhwc(&L.tmA, src.p, c.cin, src.W, src.H, B, src.ld, p.TW, p.TH, bf) ||
@@ -859,13 +836,13 @@ int build_plan(ynb_engine* e, int B, Plan** out) {
     for (int bi = 1; bi < stage_repeats()[si]; ++bi) {
       std::string u = bk + std::to_string(bi);
       Tensor o = P.T(st + "." + std::to_string(bi));
-      const int x2_off = x2_window(stage_layout(is_bf16(e), si), h, is_bf16(e) ? 8 : 4).off;
+      const int x2_off = x2_window(h, is_bf16(e) ? 8 : 4).off;
       // the previous unit's pass-through copy wrote half of x: join before reading it
       const bool ffma = e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA;
       P.pw(u + ".branch2.0", x, x2_off, mid1, 0, 1, /*join=*/ffma && bi > 1);
       if (ffma) {   // cross-check path: pass-through as a side-stream copy next to the unit's convs
         plan->net.back().mark = true;            // fork point: x is complete here
-        P.passthrough(u, x, o, h);               // o[slot(2i)] = x[i]
+        P.passthrough(u, x, o, h);               // o[2i] = x[i]
       }
       // tensor-core path: depthwise + pointwise fused, the epilogue writes whole interleaved rows (x1 | branch2)
       if (!P.dwpw(u + ".branch2.3", u + ".branch2.5", mid1, o, &x)) {
@@ -907,7 +884,7 @@ int build_plan(ynb_engine* e, int B, Plan** out) {
   for (int l = 0; l < 3; ++l) P.pw("head_det_" + std::to_string(l + 1) + ".4", head_in[l], 0, e->raw[l], 0, 1);
   // fused tail: tensor-core modes with the class counts the decode epilogue is instantiated for
   plan->fused = e->cfg.gemm_mode != YNB_GEMM_FP32_FFMA && e->cfg.num_anchors == 3 &&
-                (e->cfg.num_classes == 80 || e->cfg.num_classes == 20) && !getenv("YNB_NO_FUSED_DECODE");
+                (e->cfg.num_classes == 80 || e->cfg.num_classes == 20);
   if (plan->fused) {
     P.dst = &plan->fused_tail;
     int64_t off = 0;
@@ -1297,7 +1274,7 @@ YNB_EXPORT int ynb_forward_raw(ynb_engine* e, const float* x_dev, int32_t batch,
   float* outs[3] = {ps, pm, pl};
   for (int l = 0; l < 3; ++l) {
     const Tensor& t = e->raw[l];
-    CUDA_TRY(e, launch_nhwc_to_nchw(t.p, t.ld, t.map, outs[l], batch, t.C, t.H * t.W, e->s_main, t.es == 2));
+    CUDA_TRY(e, launch_nhwc_to_nchw(t.p, t.ld, outs[l], batch, t.C, t.H * t.W, e->s_main, t.es == 2));
   }
   if ((rc = leave(e, user))) return rc;
   return e->cfg.gemm_mode == YNB_GEMM_FP32_FFMA ? YNB_OK : check_device_error(e);
@@ -1328,9 +1305,8 @@ static int detect_ops(ynb_engine* e, Plan* plan, const float* x_dev, int batch, 
   const int64_t n = e->N();
   std::vector<Op> nms_ops(1);
   // product path: anchor-grid NMS (nms_grid.cuh); the sorted greedy NMS stays as the generic
-  // kernel (ynb_nms) and as a cross-check (YNB_NMS_SORTED=1)
-  static const bool sorted_nms = getenv("YNB_NMS_SORTED") != nullptr;
-  if (!sorted_nms && e->cfg.num_anchors == 3 && n <= 65535 && e->S % 32 == 0) {
+  // kernel (ynb_nms) and for the inputs the grid NMS does not take
+  if (e->cfg.num_anchors == 3 && n <= 65535 && e->S % 32 == 0) {
     GridNmsWorkspace gw = grid_nms_carve(e->d_nms_ws, batch, n);
     const int S = e->S;
     nms_ops[0] = {"nms(prep+build+resolve+compact)", "nms", 24.0 * batch * n * 2, 0.0, [=](cudaStream_t s2) {
@@ -1604,7 +1580,7 @@ YNB_EXPORT int ynb_read_tap(ynb_engine* e, const char* tap, int32_t batch, float
   CounterScope cs(e);
   int rc = enter(e, (cudaStream_t)stream);
   if (rc) return rc;
-  CUDA_TRY(e, launch_nhwc_to_nchw(t.p, t.ld, t.map, out_dev, batch, t.C, t.H * t.W, e->s_main, t.es == 2));
+  CUDA_TRY(e, launch_nhwc_to_nchw(t.p, t.ld, out_dev, batch, t.C, t.H * t.W, e->s_main, t.es == 2));
   return leave(e, (cudaStream_t)stream);
 }
 
@@ -1644,7 +1620,7 @@ YNB_EXPORT int ynb_dwconv3x3(const float* in, int32_t in_ld, int32_t in_off, flo
       out_step != 1 || (stride != 1 && stride != 2))
     return fail(nullptr, YNB_ERR_INVALID, "ynb_dwconv3x3: channels/ld/off must be multiples of 4, out_step 1");
   CUtensorMap tm;
-  if (!getenv("YNB_DW_NO_TMA") && make_tmap_dw(&tm, in, in_ld, in_off, batch, h_in, w_in, channels, stride)) {
+  if (make_tmap_dw(&tm, in, in_ld, in_off, batch, h_in, w_in, channels, stride)) {
     UNIT_TRY(launch_dwconv3x3_tma(tm, out, out_ld, out_off, w, b, batch, h_in, w_in, channels, stride, act,
                                   (cudaStream_t)stream));
     return YNB_OK;
@@ -1670,7 +1646,7 @@ YNB_EXPORT int ynb_pwconv(const float* in, int32_t in_ld, int32_t in_off, float*
     return fail(nullptr, YNB_ERR_INVALID, "ynb_pwconv: cin / in_ld / in_off must be multiples of 4");
   GemmParams g{};
   g.a = in; g.a_ld = in_ld; g.a_off = in_off; g.w = w; g.bias = b; g.out = out; g.out_ld = out_ld;
-  g.out_off = out_off; g.out_step = out_step; g.omap = dense_map(); g.M = pixels; g.N = cout; g.Ktot = cin;
+  g.out_off = out_off; g.out_step = out_step; g.M = pixels; g.N = cout; g.Ktot = cin;
   g.act = act;
   UNIT_TRY(launch_gemm_ffma(g, false, (cudaStream_t)stream));
   return YNB_OK;
@@ -1708,7 +1684,7 @@ YNB_EXPORT int ynb_pwconv_tc(const float* in, int32_t in_ld, int32_t in_off, flo
   p.M = pixels; p.num_tiles = (pixels + kTcBM - 1) / kTcBM; p.N = cout; p.Npad = t.Npad;
   tc_plan_tmem(p);
   p.a_box_bytes = kTcAStageBytes;
-  p.out = out; p.out_ld = out_ld; p.out_off = out_off; p.out_step = out_step; p.omap = dense_map();
+  p.out = out; p.out_ld = out_ld; p.out_off = out_off; p.out_step = out_step;
   p.bias = b_dev; p.act = act; p.err_flag = d_err;
   long long* d_trace = nullptr;
   const int trace_cap = 8 * 64 * 32;     // (role, local tile, step) slots, see YNB_TRACE
@@ -1718,7 +1694,7 @@ YNB_EXPORT int ynb_pwconv_tc(const float* in, int32_t in_ld, int32_t in_off, flo
     UNIT_TRY(cudaMemset(d_trace, 0, (1 + 4 * trace_cap) * 8));
     p.trace = d_trace; p.trace_cap = trace_cap;
   }
-  p.tma_store = (out_step == 1 && out_off % 4 == 0 && getenv("YNB_TC_NO_TMA_STORE") == nullptr) ? 1 : 0;
+  p.tma_store = (out_step == 1 && out_off % 4 == 0) ? 1 : 0;
   if (getenv("YNB_TC_PASS") != nullptr && cin >= cout && out_ld >= 2 * cout) {
     // timeline hook for the interleave epilogue: pass-through = first `cout` channels of the input rows
     p.pass = in; p.pass_ld = in_ld; p.tma_store = 0; p.out_off = 1; p.out_step = 2;
@@ -1742,8 +1718,8 @@ YNB_EXPORT int ynb_pwconv_tc(const float* in, int32_t in_ld, int32_t in_off, flo
       cudaMemcpy(h.data(), d_trace, h.size() * 8, cudaMemcpyDeviceToHost);
       int n = 0;
       for (int i = 0; i < trace_cap; ++i) n += h[4 + 4 * i] != 0;
-      fprintf(stderr, "YNB_TC_TRACE stages=%d resident=%d nmain=%d acc_stages=%d steps=%d grid=%u events=%d\n",
-              p.num_stages, p.w_resident, p.nmain, p.acc_stages, p.num_steps, L.grid, n);
+      fprintf(stderr, "YNB_TC_TRACE stages=%d resident=%d nacc=%d acc_stages=%d steps=%d grid=%u events=%d\n",
+              p.num_stages, p.w_resident, p.nacc, p.acc_stages, p.num_steps, L.grid, n);
       for (int i = 0; i < trace_cap; ++i)
         if (h[4 + 4 * i] != 0)
           fprintf(stderr, "TRACE %lld %lld %lld %lld\n", h[1 + 4 * i], h[2 + 4 * i], h[3 + 4 * i], h[4 + 4 * i]);
@@ -1791,7 +1767,7 @@ YNB_EXPORT int ynb_dwpw_tc(const float* in, int32_t in_ld, const float* dw_w, co
   DwPwParams& p = L.p;
   memset(&p, 0, sizeof(p));
   p.dw_w = dw_w; p.dw_b = dw_b; p.dw_act = dw_act;
-  p.out = out; p.out_ld = out_ld; p.out_off = 0; p.omap = dense_map();
+  p.out = out; p.out_ld = out_ld; p.out_off = 0;
   p.bias = pw_b; p.act = act; p.pass = pass; p.pass_ld = pass ? pass_ld : 0; p.err_flag = d_err;
   long long* d_trace = nullptr;
   const bool want_trace = getenv("YNB_DP_TRACE") != nullptr;
@@ -1989,8 +1965,7 @@ YNB_EXPORT int ynb_dwconv3x3_bwd_data(const float* dout, int32_t do_ld, int32_t 
   const bool vec = channels % 4 == 0 && do_ld % 4 == 0 && do_off % 4 == 0 && di_ld % 4 == 0 && di_off % 4 == 0 &&
                    ((uintptr_t)dout | (uintptr_t)din | (uintptr_t)w) % 16 == 0;
   CUtensorMap tm;
-  if (stride == 1 && vec && !getenv("YNB_DW_NO_TMA") &&
-      make_tmap_dw(&tm, dout, do_ld, do_off, batch, h_in, w_in, channels, 1)) {
+  if (stride == 1 && vec && make_tmap_dw(&tm, dout, do_ld, do_off, batch, h_in, w_in, channels, 1)) {
     // stride 1: the forward convolution of d_out with the taps reversed, on the TMA halo-tile kernel
     UNIT_TRY(launch_dwconv3x3_tma(tm, din, di_ld, di_off, w, nullptr, batch, h_in, w_in, channels, 1, YNB_ACT_NONE, st,
                                   /*reversed_taps=*/true));
@@ -2049,8 +2024,6 @@ YNB_EXPORT int ynb_dwconv3x3_bwd_weight(const float* dout, int32_t do_ld, int32_
   return YNB_OK;
 }
 
-static bool pw_wgrad_use_tc(int cin) { return wgrad_tc_kpad(cin) != 0 && !getenv("YNB_PWBW_FFMA"); }
-
 YNB_EXPORT int64_t ynb_pwconv_bwd_weight_workspace_bytes(int64_t pixels, int32_t cin, int32_t cout) {
   int64_t floats = (int64_t)pw_bwd_chunks(pixels, cin, cout) * ((int64_t)cout * cin + cout);
   if (wgrad_tc_kpad(cin)) floats = std::max<int64_t>(floats, wgrad_tc_partial_floats(pixels, cin, cout));
@@ -2065,7 +2038,7 @@ YNB_EXPORT int ynb_pwconv_bwd_weight(const float* dout, int32_t do_ld, int32_t d
     return fail(nullptr, YNB_ERR_INVALID, "ynb_pwconv_bwd_weight: bad arguments / workspace too small");
   const bool aligned = cin % 4 == 0 && cout % 4 == 0 && do_ld % 4 == 0 && do_off % 4 == 0 && in_ld % 4 == 0 &&
                        in_off % 4 == 0 && ((uintptr_t)dout | (uintptr_t)in) % 16 == 0;
-  if (pw_wgrad_use_tc(cin) && aligned) {
+  if (wgrad_tc_kpad(cin) != 0 && aligned) {
     // tcgen05 path (3xTF32 = fp32 parity): pixels are the contraction dimension
     cudaStream_t st = (cudaStream_t)stream;
     const int chunks = wgrad_tc_chunks(pixels, cout);
@@ -2097,10 +2070,8 @@ YNB_EXPORT int ynb_pwconv_bwd_weight(const float* dout, int32_t do_ld, int32_t d
   float* pb = pw + (long long)chunks * cout * cin;
   cudaStream_t st = (cudaStream_t)stream;
   // a chunk past the end of M (rounding of m_per_chunk) writes zeros: no memset needed
-  const int vec = cin % 4 == 0 && cout % 4 == 0 && do_ld % 4 == 0 && do_off % 4 == 0 && in_ld % 4 == 0 &&
-                  in_off % 4 == 0 && ((uintptr_t)dout | (uintptr_t)in) % 16 == 0;
   dim3 grid(chunks, (cout + kPwBwdTile - 1) / kPwBwdTile, (cin + kPwBwdTile - 1) / kPwBwdTile);
-  if (vec && !getenv("YNB_PWBW_NO_ASYNC")) {
+  if (aligned) {
     // per device, cheap: set on every call (one process may drive several devices)
     UNIT_TRY(cudaFuncSetAttribute(pwconv_bwd_weight_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)kPwBwdAsyncSmem));
@@ -2108,7 +2079,7 @@ YNB_EXPORT int ynb_pwconv_bwd_weight(const float* dout, int32_t do_ld, int32_t d
                                                                        pixels, cin, cout, m_per_chunk);
   } else {
     pwconv_bwd_weight_kernel<<<grid, 256, 0, st>>>(dout, do_ld, do_off, in, in_ld, in_off, pw, pb, pixels, cin, cout,
-                                                   m_per_chunk, vec);
+                                                   m_per_chunk);
   }
   YNB_COUNT_LAUNCH();
   launch_reduce_partials(pw, chunks, (long long)cout * cin, dw, st);
@@ -2378,7 +2349,7 @@ YNB_EXPORT int ynb_conv3x3_tc(const float* in, int32_t in_ld, float* out, int32_
   p.N = cout; p.Npad = t.Npad;
   tc_plan_tmem(p);
   p.a_box_bytes = (uint32_t)(p.TH * p.TW * 128);
-  p.out = out; p.out_ld = out_ld; p.out_off = 0; p.out_step = 1; p.omap = dense_map();
+  p.out = out; p.out_ld = out_ld; p.out_off = 0; p.out_step = 1;
   p.bias = b_dev; p.act = act; p.err_flag = d_err;
   if (!make_tmap_2d(&t.tm_hi, t.hi, t.Kpad, t.Npad, t.Kpad, t.Npad) ||
       !make_tmap_2d(&t.tm_lo, t.lo, t.Kpad, t.Npad, t.Kpad, t.Npad) ||
@@ -2461,7 +2432,7 @@ YNB_EXPORT int ynb_pwconv_tc_async(const float* in, int32_t in_ld, int32_t in_of
   p.M = pixels; p.num_tiles = (pixels + kTcBM - 1) / kTcBM; p.N = cout; p.Npad = t.Npad;
   tc_plan_tmem(p);
   p.a_box_bytes = kTcAStageBytes;
-  p.out = out; p.out_ld = out_ld; p.out_off = out_off; p.out_step = out_step; p.omap = dense_map();
+  p.out = out; p.out_ld = out_ld; p.out_off = out_off; p.out_step = out_step;
   p.bias = b_dev; p.act = act; p.err_flag = a.flag;
   p.tma_store = (out_step == 1 && out_off % 4 == 0) ? 1 : 0;
   if (!make_tmap_2d(&t.tm_hi, t.hi, t.Kpad, t.Npad, t.Kpad, t.Npad) ||
@@ -2509,7 +2480,7 @@ YNB_EXPORT int ynb_conv3x3_tc_async(const float* in, int32_t in_ld, float* out, 
   p.N = cout; p.Npad = t.Npad;
   tc_plan_tmem(p);
   p.a_box_bytes = (uint32_t)(p.TH * p.TW * 128);
-  p.out = out; p.out_ld = out_ld; p.out_off = 0; p.out_step = 1; p.omap = dense_map();
+  p.out = out; p.out_ld = out_ld; p.out_off = 0; p.out_step = 1;
   p.bias = b_dev; p.act = act; p.err_flag = a.flag;
   if (!make_tmap_2d(&t.tm_hi, t.hi, t.Kpad, t.Npad, t.Kpad, t.Npad) ||
       !make_tmap_2d(&t.tm_lo, t.lo, t.Kpad, t.Npad, t.Kpad, t.Npad) ||
