@@ -265,6 +265,43 @@ int  ynb_voc_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num_classes, 
                   int32_t* order_dev, int8_t* flags_dev, void* workspace_dev, int64_t workspace_bytes,
                   void* stream);
 
+/* COCO bbox AP on the device (evaluator/cocoapi_evaluator.py: the results JSON, then pycocotools'
+ * COCOeval(cocoGt, cocoDt, 'bbox') evaluate + accumulate with the bbox defaults T = 10 IoU thresholds, R = 101 recall
+ * thresholds, A = 4 area ranges [0, 1e10], [0, 32^2], [32^2, 96^2], [96^2, 1e10] (bounds inclusive), M = maxDets
+ * {1, 10, 100}).
+ *
+ * ynb_coco_append turns the kept rows of a batch (after ynb_map_boxes) into results entries, one int32 row each:
+ *     rows_dev[slot] = {image_base + b, class, score bits, x1, y1, x2, y2 bits}
+ * the raw float32 values (bbox = [x1, y1, x2 - x1, y2 - y1] in float64, as the Python floats of the JSON).  Slots,
+ * state_dev and the capacity as ynb_voc_append; state_dev[1] counts rejected values (class out of range, non-finite
+ * score or box). */
+int  ynb_coco_append(const float* boxes_dev, const float* scores_dev, const int32_t* cls_dev,
+                     const int32_t* counts_dev, int32_t batch, int64_t n_per_image, int32_t image_base,
+                     int32_t num_classes, int32_t* rows_dev, int64_t capacity, int64_t* state_dev, void* stream);
+
+/* COCOeval over rows_dev[0, n_rows).  Image i of the rows (its add index) is evaluated at image_rank_dev[i], its
+ * position among the sorted image ids; class c maps to category index class_cat_dev[c] into the sorted GT category
+ * ids (-1: dropped, as loadRes results of a non-GT category are).  GT of the evaluated images and categories, in
+ * annotation-file order and bucketed by cell (rank, k): cell (i, k) is [gt_start_dev[i * num_cats + k],
+ * gt_start_dev[i * num_cats + k + 1]), with gt_boxes_dev [G][4] float64 xywh, gt_area_dev [G] (the annotations'
+ * area field) and gt_crowd_dev [G]; annotation ids must be positive.  iou_thrs [10] and rec_thrs [101] are HOST
+ * arrays (np.linspace as Params builds them).
+ *   Per cell: detections by score descending (ties in file order), the first 100; bbIou in float64 (crowd GT: the
+ *   detection's area as the union); per range and threshold the greedy scan of evaluateImg (non-ignored GT first,
+ *   IoU >= min(t, 1 - 1e-10), the later GT on equal IoU, matched non-crowd GT skipped).  Per (category, range,
+ *   maxDet): the first maxDet of every cell in ascending image rank, stable-sorted by score; tp / fp cumsums with
+ *   ignored detections counting in neither; rc = tp / npig, pr = tp / ((fp + tp) + 2^-52), its suffix maximum,
+ *   q[r] = pr[searchsorted(rc, rec_thrs[r], 'left')], 0 past the end.
+ * Outputs precision_dev [10][101][num_cats][4][3] and recall_dev [10][num_cats][4][3] float64, -1 where the
+ * (category, range) has no non-ignored GT.  Deterministic. */
+int64_t ynb_coco_eval_workspace_bytes(int64_t n_rows, int32_t num_images, int32_t num_cats, int64_t n_gt);
+int  ynb_coco_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num_classes, int32_t num_images,
+                   const int32_t* image_rank_dev, const int32_t* class_cat_dev, int32_t num_cats,
+                   const double* gt_boxes_dev, const double* gt_area_dev, const uint8_t* gt_crowd_dev,
+                   const int32_t* gt_start_dev, int64_t n_gt, const double* iou_thrs, const double* rec_thrs,
+                   double* precision_dev, double* recall_dev, void* workspace_dev, int64_t workspace_bytes,
+                   void* stream);
+
 /* Pointwise 1x1 conv = GEMM over pixels, + bias + activation, fp32 FFMA variant
  * (backbone/shufflenetv2.py:46,54,60; utils/modules.py:11 with k=1).
  * w_dev is [cout][cin] row-major, b_dev [cout].

@@ -27,6 +27,7 @@
 #include "train_ops.cuh"
 #include "wgrad_tc.cuh"
 #include "voc_eval.cuh"
+#include "coco_eval.cuh"
 #include "topology.h"
 
 #define YNB_EXPORT extern "C" __attribute__((visibility("default")))
@@ -1509,6 +1510,55 @@ YNB_EXPORT int ynb_voc_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num
                                             gt_difficult_dev, gt_start_dev, n_gt, ovthresh, use_07_metric ? 1 : 0,
                                             ap_dev, npos_dev, order_dev, flags_dev, w, (cudaStream_t)stream);
   if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("voc_eval: ") + cudaGetErrorString(r));
+  return YNB_OK;
+}
+
+YNB_EXPORT int ynb_coco_append(const float* boxes_dev, const float* scores_dev, const int32_t* cls_dev,
+                               const int32_t* counts_dev, int32_t batch, int64_t n_per_image, int32_t image_base,
+                               int32_t num_classes, int32_t* rows_dev, int64_t capacity, int64_t* state_dev,
+                               void* stream) {
+  if (!boxes_dev || !scores_dev || !cls_dev || !counts_dev || !rows_dev || !state_dev || batch <= 0 ||
+      n_per_image <= 0 || image_base < 0 || (int64_t)image_base + batch > INT32_MAX || num_classes < 1 ||
+      num_classes > kVocMaxClasses || capacity < 0 || capacity > kVocMaxRows)
+    return fail(nullptr, YNB_ERR_INVALID, "ynb_coco_append: bad arguments");
+  cudaError_t r = ynb::coco::launch_coco_append(boxes_dev, scores_dev, cls_dev, counts_dev, batch, n_per_image,
+                                                image_base, num_classes, rows_dev, capacity,
+                                                reinterpret_cast<long long*>(state_dev), (cudaStream_t)stream);
+  if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("coco_append: ") + cudaGetErrorString(r));
+  return YNB_OK;
+}
+
+// Sort keys are uint32 and cell keys image_rank * K + k: the cell count stays below 2^31.
+YNB_EXPORT int64_t ynb_coco_eval_workspace_bytes(int64_t n_rows, int32_t num_images, int32_t num_cats,
+                                                 int64_t n_gt) {
+  if (n_rows < 0 || n_rows > kVocMaxRows || num_images < 0 || num_cats < 1 || num_cats > kVocMaxClasses ||
+      (int64_t)num_images * num_cats >= INT32_MAX || n_gt < 0 || n_gt >= INT32_MAX)
+    return -1;
+  return ynb::coco::eval_workspace(nullptr, n_rows, (int64_t)num_images * num_cats, num_cats, n_gt, nullptr);
+}
+
+YNB_EXPORT int ynb_coco_eval(const int32_t* rows_dev, int64_t n_rows, int32_t num_classes, int32_t num_images,
+                             const int32_t* image_rank_dev, const int32_t* class_cat_dev, int32_t num_cats,
+                             const double* gt_boxes_dev, const double* gt_area_dev, const uint8_t* gt_crowd_dev,
+                             const int32_t* gt_start_dev, int64_t n_gt, const double* iou_thrs,
+                             const double* rec_thrs, double* precision_dev, double* recall_dev, void* workspace_dev,
+                             int64_t workspace_bytes, void* stream) {
+  const int64_t need = ynb_coco_eval_workspace_bytes(n_rows, num_images, num_cats, n_gt);
+  if (need < 0 || num_classes < 1 || num_classes > kVocMaxClasses || (n_rows > 0 && num_images < 1) ||
+      (n_rows > 0 && (!rows_dev || !image_rank_dev)) || !class_cat_dev ||
+      (n_gt > 0 && (!gt_boxes_dev || !gt_area_dev || !gt_crowd_dev)) || !gt_start_dev || !iou_thrs || !rec_thrs ||
+      !precision_dev || !recall_dev || !workspace_dev || workspace_bytes < need)
+    return fail(nullptr, YNB_ERR_INVALID, "ynb_coco_eval: bad arguments / workspace too small");
+  ynb::coco::Thresholds thr;
+  for (int i = 0; i < ynb::coco::kT; ++i) thr.iou[i] = iou_thrs[i];
+  for (int i = 0; i < ynb::coco::kR; ++i) thr.rec[i] = rec_thrs[i];
+  ynb::coco::EvalWorkspace w;
+  ynb::coco::eval_workspace(workspace_dev, n_rows, (int64_t)num_images * num_cats, num_cats, n_gt, &w);
+  cudaError_t r = ynb::coco::launch_coco_eval(rows_dev, n_rows, num_classes, num_images, image_rank_dev,
+                                              class_cat_dev, num_cats, gt_boxes_dev, gt_area_dev, gt_crowd_dev,
+                                              gt_start_dev, n_gt, thr, precision_dev, recall_dev, w,
+                                              (cudaStream_t)stream);
+  if (r != cudaSuccess) return fail(nullptr, YNB_ERR_CUDA, std::string("coco_eval: ") + cudaGetErrorString(r));
   return YNB_OK;
 }
 

@@ -397,6 +397,40 @@ class YOLONano(nn.Module):
             run(batch)
         return dets.evaluate(gt, ovthresh=ovthresh, use_07_metric=use_07_metric)
 
+    def evaluate_coco(self, samples, gt, class_ids, batch_size: int = 64, capacity: Optional[int] = None):
+        """`COCOAPIEvaluator.evaluate` (evaluator/cocoapi_evaluator.py) on the device: `samples` is an iterable of
+        (ORIGINAL uint8 BGR image, COCO image id), what `COCODataset.pull_image(i)` returns; `gt` the instances JSON
+        as a dict (`dataset.coco.dataset`); `class_ids` the dataset's class_ids.  Per batch: ValTransforms,
+        detection, the inverse box mapping and the results entries stay on the device; the host waits once, for the
+        precision and recall arrays.  Returns COCOeval's 12 stats (float64 [12]): the reference's (ap50, ap50_95)
+        are stats[1] and stats[0].  `capacity` bounds the results entries (default: every anchor box of every GT
+        image, which cannot overflow for distinct GT image ids)."""
+        from .coco_eval import COCODetections
+        if batch_size < 1:
+            raise ValueError("batch_size must be positive")
+        eng = self.engine(batch_size)
+        if capacity is None:
+            capacity = len(gt["images"]) * eng.num_boxes
+        dets = COCODetections(eng.device, self.num_classes, capacity)
+        batch, ids = [], []
+
+        def run(batch):
+            eng = self.engine(len(batch))
+            x, maps = eng.preprocess_images(batch)
+            boxes, scores, cls, counts = eng.forward_detect(x)
+            eng.map_boxes(boxes, counts, maps)
+            dets.add(boxes, scores, cls, counts)
+
+        for im, image_id in samples:
+            batch.append(im)
+            ids.append(int(image_id))
+            if len(batch) == batch_size:
+                run(batch)
+                batch = []
+        if batch:
+            run(batch)
+        return dets.evaluate(gt, ids, class_ids)
+
     def forward(self, x, target=None):
         if self.trainable:
             # training branch (models/yolo_nano.py:333-358).  The returned losses are plain device scalars WITHOUT a
